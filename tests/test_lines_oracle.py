@@ -25,10 +25,10 @@ def _images():
            ("lines640", synth.make_line_image(1)), ("lines752", synth.make_line_image(2, 480, 752)),
            ("noise", np.random.default_rng(5).integers(0, 256, (480, 640), dtype=np.uint8)),
            ("flat", np.full((480, 640), 77, np.uint8))]
-    for f in ("equirectangular_image_001.jpg", "equirectangular_image_002.jpg"):
-        p = Path("/root/reference/test/data") / f   # only present in the authoring container
-        if p.exists():
-            out.append((f, cv2.resize(cv2.imread(str(p), cv2.IMREAD_GRAYSCALE), (640, 480))))
+    # the reference's test/data/equirectangular_image_00{1,2}.jpg at 640x480, central 240 rows (tools/gen_golden.py)
+    for i in (1, 2):
+        f = f"equirectangular_image_00{i}_band.png"
+        out.append((f, cv2.imread(str(ROOT / "tests" / "golden" / f), cv2.IMREAD_GRAYSCALE)))
     return out
 
 

@@ -7,7 +7,17 @@ cv2_primitives.npz  cv::resize / cv::FAST / cv::GaussianBlur 7x7 + 5x5 / cv::Sob
 cv2_lsd.npz         cv::LineSegmentDetector(1, 0.5, 0.6, 2, 22.5, 1, 0.6, 1024) segments on two seeded images
 orb_mirror.npz      orb_extractor::extract with every third-party stage done by cv2 (tests/test_orb_oracle.py mirror)
 line_extract.npz    LineFeatureTracker::extract_LSD_LBD output of the oracle (whose LSD stage is pinned to cv2 above)
-The images are regenerated from their seeds by the tests; only the outputs are stored."""
+The images are regenerated from their seeds by the tests; only the outputs are stored.
+
+    python tools/gen_golden.py --reference <Structure-PLP-SLAM source tree>
+
+writes, instead, the fixtures taken from the reference's own data files (too large to store whole):
+orb_vocab_sample.npz  orb_vocab/orb_vocab.dbow2: its header, every node a descent of the 16 test descriptors visits or
+                      compares against (the children of each node on their paths), and transform()'s answers on the
+                      whole file
+equirectangular_image_00{1,2}_band.png
+                      test/data/equirectangular_image_00{1,2}.jpg, grayscale, resized to 640x480, rows 120-359"""
+import argparse
 import sys
 from pathlib import Path
 
@@ -16,6 +26,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT / "tests"))
+import bow_data  # noqa: E402
 import oracle_api  # noqa: E402
 import synth  # noqa: E402
 import test_orb_oracle  # noqa: E402
@@ -23,9 +34,56 @@ import test_orb_oracle  # noqa: E402
 OUT = ROOT / "tests" / "golden"
 
 
+def reference_fixtures(ref: Path, orc):
+    # ---- the shipped vocabulary, pruned to the subtree the test descents touch
+    path = ref / "orb_vocab" / "orb_vocab.dbow2"
+    raw = np.fromfile(path, np.uint8)
+    header, rec = raw[:24].copy(), raw[24:].reshape(-1, 41)
+    vocab = dict(k=10, L=6, parent=rec[:, :4].copy().view("<i4").ravel(), desc=rec[:, 4:36],
+                 weight=rec[:, 36:40].copy().view("<f4").ravel(), is_leaf=rec[:, 40])
+    rng = np.random.default_rng(0)
+    queries = np.concatenate([synth.rand_desc(rng, 8),
+                              synth.flip_bits(rng, vocab["desc"][rng.integers(0, len(rec), 8)], 12)])
+    v = orc.bow_vocab_load(path)
+    info = orc.bow_vocab_info(v)
+    word, node, w = orc.bow_transform(v, queries, 4)
+    orc.bow_vocab_destroy(v)
+    assert [(int(a), int(b), float(c)) for a, b, c in zip(word, node, w)] == bow_data.transform_numpy(vocab, queries, 4)
+    n_nodes = len(vocab["parent"]) + 1
+    by_parent = np.argsort(vocab["parent"], kind="stable") + 1                 # node ids, grouped by parent, file order
+    first_child = np.searchsorted(vocab["parent"][by_parent - 1], np.arange(n_nodes + 1))
+    bits = np.unpackbits(vocab["desc"], axis=1)
+    keep = set()
+    for q in np.unpackbits(queries, axis=1):
+        cur = 0
+        while first_child[cur] < first_child[cur + 1]:
+            ch = by_parent[first_child[cur]:first_child[cur + 1]]
+            keep.update(ch.tolist())
+            cur = int(ch[np.argmin((bits[ch - 1] != q).sum(1))])
+    ids = np.array(sorted(keep), np.int32)
+    word_of = np.cumsum(vocab["is_leaf"], dtype=np.int64) - 1
+    np.savez_compressed(OUT / "orb_vocab_sample.npz", header=header,
+                        info=np.array([info["k"], info["L"], info["num_nodes"], info["num_words"]], np.int32),
+                        ids=ids, parent=vocab["parent"][ids - 1], desc=vocab["desc"][ids - 1],
+                        weight=vocab["weight"][ids - 1], is_leaf=vocab["is_leaf"][ids - 1],
+                        word_id=np.where(vocab["is_leaf"][ids - 1] > 0, word_of[ids - 1], -1).astype(np.int32),
+                        queries=queries, word=word, node=node, node_weight=w)
+    # ---- the reference's test images at the resolution of the LSD tests; the central band keeps the file small
+    for i in (1, 2):
+        img = cv2.imread(str(ref / "test" / "data" / f"equirectangular_image_00{i}.jpg"), cv2.IMREAD_GRAYSCALE)
+        cv2.imwrite(str(OUT / f"equirectangular_image_00{i}_band.png"), cv2.resize(img, (640, 480))[120:360],
+                    [cv2.IMWRITE_PNG_COMPRESSION, 9])
+
+
 def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reference", type=Path, default=None, help="Structure-PLP-SLAM source tree")
+    args = ap.parse_args()
     OUT.mkdir(exist_ok=True)
     orc = oracle_api.Oracle()
+    if args.reference is not None:
+        reference_fixtures(args.reference, orc)
+        return
     tex = synth.make_texture(4321, 240, 320, n_rect=120, n_blob=500)      # the image of __graft_entry__.smoke()
     lines = synth.make_line_image(7, 240, 320, n_patch=16)
     # ---- third-party primitives
