@@ -38,15 +38,6 @@ struct plp_ba {
 
 namespace {
 
-struct Carver {
-    size_t off = 0;
-    size_t take(size_t bytes) {
-        const size_t o = off;
-        off += (bytes + 255) & ~(size_t)255;
-        return o;
-    }
-};
-
 // One LM try = a fixed sequence of 7 launches whose arguments never change (all state lives in device memory),
 // so it is captured once into a CUDA graph and replayed: ~7 x 4 us of launch overhead -> one graph launch.
 plp_status launch_try(plp_ba *b) {
@@ -249,72 +240,109 @@ plp_status plp_ba_create(plp_ctx *ctx, const plp_ba_problem *p, const plp_ba_cfg
     b->n_lines = n_lines;
     b->n_pe = n_pe;
     b->n_le = n_le;
-    // ---- carve one device block
-    Carver cv;
+    // ---- lay out one device block
+    BaDev &D = b->dev;
+    memset(&D, 0, sizeof(D));
+    Layout lay;
     const size_t P1 = std::max(n_pts, 1), L1 = std::max(n_lines, 1), E1 = std::max(n_pe, 1), F1 = std::max(n_le, 1);
-    const size_t o_hidx = cv.take(n_kf * 4), o_pose0 = cv.take(n_kf * sizeof(se3::Pose)), o_pose1 = cv.take(n_kf * sizeof(se3::Pose));
-    const size_t o_pert = cv.take((size_t)n_kf * 12 * sizeof(se3::Pose));
-    const size_t o_pbi = cv.take(n_pairs * 4), o_pbj = cv.take(n_pairs * 4);
-    const size_t o_pts0 = cv.take(P1 * 24), o_pts1 = cv.take(P1 * 24), o_ln0 = cv.take(L1 * 48), o_ln1 = cv.take(L1 * 48);
-    const size_t o_ptoff = cv.take((P1 + 1) * 4), o_ptkf = cv.take(E1 * 4), o_ptlm = cv.take(E1 * 4), o_ptobs = cv.take(E1 * 12);
-    const size_t o_ptinfo = cv.take(E1 * 4), o_ptlvl = cv.take(E1), o_ptout = cv.take(E1), o_ptchi = cv.take(E1 * 8);
-    const size_t o_ptW = cv.take(E1 * 24 * 8), o_ptD = cv.take(P1 * 16 * 8), o_ptbl = cv.take(P1 * 4 * 8), o_ptact = cv.take(P1);
-    const size_t o_ptplane = cv.take(P1 * 4), o_plfn = cv.take((size_t)std::max(p->n_plane_edges, 1) * 32);
-    const size_t o_plerr = cv.take((size_t)std::max(p->n_plane_edges, 1) * 8);
-    const size_t o_lnoff = cv.take((L1 + 1) * 4), o_lnkf = cv.take(F1 * 4), o_lnlm = cv.take(F1 * 4), o_lnobs = cv.take(F1 * 16);
-    const size_t o_lninfo = cv.take(F1 * 4), o_lnlvl = cv.take(F1), o_lnout = cv.take(F1), o_lnchi = cv.take(F1 * 8);
-    const size_t o_lnW = cv.take(F1 * 24 * 8), o_lnD = cv.take(L1 * 16 * 8), o_lnbl = cv.take(L1 * 4 * 8), o_lnact = cv.take(L1);
-    const size_t o_ranges = cv.take((G + 1) * 4), o_partial = cv.take(large ? 64 : (size_t)G * packed_len * 8);
-    const size_t o_dense = cv.take(large ? ba_dense_bytes(n_free) : 64);
-    const size_t o_packed = cv.take((size_t)(packed_sum_len + world + 8) * 8), o_dp = cv.take((size_t)6 * std::max(n_free, kBaMaxFree) * 8);
-    const size_t o_tp = cv.take((size_t)G * 16), o_ts = cv.take(64), o_state = cv.take(sizeof(BaState));
-    const size_t o_Tin = cv.take(n_kf * 128), o_ptsin = cv.take(P1 * 24), o_lnin = cv.take(L1 * 48), o_Tout = cv.take(n_kf * 128);
-    const size_t o_ptsout = cv.take(P1 * 24), o_lnout2 = cv.take(L1 * 48), o_stop = cv.take(64);
-    if (cudaMalloc((void **)&b->d_block, cv.off) != cudaSuccess) {
-        set_error("local BA: cudaMalloc(%zu) failed", cv.off);
+    const size_t PL1 = std::max(p->n_plane_edges, 1);
+    lay.out(D.kf_hidx, n_kf);
+    lay.out(D.poses[0], n_kf);
+    lay.out(D.poses[1], n_kf);
+    lay.out(D.pert_pose, (size_t)n_kf * 12);
+    lay.out(D.pair_bi, n_pairs);
+    lay.out(D.pair_bj, n_pairs);
+    lay.out(D.pts[0], P1 * 3);
+    lay.out(D.pts[1], P1 * 3);
+    lay.out(D.lines[0], L1 * 6);
+    lay.out(D.lines[1], L1 * 6);
+    lay.out(D.pt_off, P1 + 1);
+    lay.out(D.pt_kf, E1);
+    lay.out(D.pt_lm, E1);
+    lay.out(D.pt_obs, E1 * 3);
+    lay.out(D.pt_info, E1);
+    lay.out(D.pt_level, E1);
+    lay.out(D.pt_outlier, E1);
+    lay.out(D.pt_chi2, E1);
+    lay.out(D.pt_W, E1 * 24);
+    lay.out(D.pt_Dinv, P1 * 16);
+    lay.out(D.pt_bl, P1 * 4);
+    lay.out(D.pt_active, P1);
+    lay.out(D.pt_plane, P1);
+    lay.out(D.pl_fn, PL1 * 4);
+    lay.out(D.pl_err, PL1);
+    lay.out(D.ln_off, L1 + 1);
+    lay.out(D.ln_kf, F1);
+    lay.out(D.ln_lm, F1);
+    lay.out(D.ln_obs, F1 * 4);
+    lay.out(D.ln_info, F1);
+    lay.out(D.ln_level, F1);
+    lay.out(D.ln_outlier, F1);
+    lay.out(D.ln_chi2, F1);
+    lay.out(D.ln_W, F1 * 24);
+    lay.out(D.ln_Dinv, L1 * 16);
+    lay.out(D.ln_bl, L1 * 4);
+    lay.out(D.ln_active, L1);
+    lay.out(D.cta_ranges, (size_t)G + 1);
+    lay.out(D.partial, large ? 8 : (size_t)G * packed_len);
+    lay.out(D.dense, large ? ba_dense_bytes(n_free) / 8 : 8);
+    lay.out(D.packed, (size_t)packed_sum_len + world + 8);
+    lay.out(D.dp, (size_t)6 * std::max(n_free, kBaMaxFree));
+    lay.out(D.trial_partial, (size_t)G * 2);
+    lay.out(D.trial_sum, 8);
+    lay.out(D.state, 1);
+    lay.out(b->d_T_in, (size_t)n_kf * 16);
+    lay.out(b->d_pts_in, P1 * 3);
+    lay.out(b->d_lines_in, L1 * 6);
+    lay.out(b->d_T_out, (size_t)n_kf * 16);
+    lay.out(b->d_pts_out, P1 * 3);
+    lay.out(b->d_lines_out, L1 * 6);
+    lay.out(b->d_stop, 8);
+    if (cudaMalloc((void **)&b->d_block, lay.bytes()) != cudaSuccess) {
+        set_error("local BA: cudaMalloc(%zu) failed", lay.bytes());
         delete b;
         return PLP_ERR_CUDA;
     }
-    b->block_bytes = cv.off;
+    b->block_bytes = lay.bytes();
+    lay.bind(b->d_block);
     if (cudaMallocHost((void **)&b->h_state, sizeof(BaState)) != cudaSuccess ||
         cudaMallocHost((void **)&b->h_stop, 16) != cudaSuccess) {
         set_error("local BA: cudaMallocHost failed");
         plp_ba_destroy(b);
         return PLP_ERR_CUDA;
     }
-    uint8_t *d = b->d_block;
-    cudaError_t up_err = cudaMemsetAsync(d, 0, cv.off, ctx->stream);
-    auto up = [&](size_t off, const void *src, size_t bytes) {
-        if (bytes && up_err == cudaSuccess) up_err = cudaMemcpyAsync(d + off, src, bytes, cudaMemcpyHostToDevice, ctx->stream);
+    cudaError_t up_err = cudaMemsetAsync(b->d_block, 0, lay.bytes(), ctx->stream);
+    auto up = [&](const auto *dst, const auto *src, size_t n) {
+        static_assert(std::is_same<std::decay_t<decltype(*dst)>, std::decay_t<decltype(*src)>>::value, "types differ");
+        if (n && up_err == cudaSuccess)
+            up_err = cudaMemcpyAsync((void *)dst, src, n * sizeof(*src), cudaMemcpyHostToDevice, ctx->stream);
     };
-    up(o_hidx, hidx.data(), n_kf * 4);
-    up(o_pbi, pair_bi.data(), n_pairs * 4);
-    up(o_pbj, pair_bj.data(), n_pairs * 4);
-    up(o_ptoff, pt_off.data(), (n_pts + 1) * 4);
-    up(o_ptkf, p->pt_edge_kf, (size_t)n_pe * 4);
-    up(o_ptlm, p->pt_edge_lm, (size_t)n_pe * 4);
-    up(o_ptobs, p->pt_edge_obs, (size_t)n_pe * 12);
-    up(o_ptinfo, p->pt_edge_inv_sigma_sq, (size_t)n_pe * 4);
-    up(o_ptplane, pt_plane.data(), (size_t)n_pts * 4);
-    up(o_plfn, p->plane_edge_fn, (size_t)p->n_plane_edges * 32);
-    up(o_lnoff, ln_off.data(), (n_lines + 1) * 4);
-    up(o_lnkf, p->line_edge_kf, (size_t)n_le * 4);
-    up(o_lnlm, p->line_edge_lm, (size_t)n_le * 4);
-    up(o_lnobs, p->line_edge_obs, (size_t)n_le * 16);
-    up(o_lninfo, p->line_edge_inv_sigma_sq, (size_t)n_le * 4);
-    up(o_ranges, ranges.data(), (G + 1) * 4);
-    up(o_Tin, p->kf_pose_cw, (size_t)n_kf * 128);
-    up(o_ptsin, p->pt_pos_w, (size_t)n_pts * 24);
-    up(o_lnin, p->line_plucker, (size_t)n_lines * 48);
+    up(D.kf_hidx, hidx.data(), n_kf);
+    up(D.pair_bi, pair_bi.data(), n_pairs);
+    up(D.pair_bj, pair_bj.data(), n_pairs);
+    up(D.pt_off, pt_off.data(), (size_t)n_pts + 1);
+    up(D.pt_kf, p->pt_edge_kf, n_pe);
+    up(D.pt_lm, p->pt_edge_lm, n_pe);
+    up(D.pt_obs, p->pt_edge_obs, (size_t)n_pe * 3);
+    up(D.pt_info, p->pt_edge_inv_sigma_sq, n_pe);
+    up(D.pt_plane, pt_plane.data(), n_pts);
+    up(D.pl_fn, p->plane_edge_fn, (size_t)p->n_plane_edges * 4);
+    up(D.ln_off, ln_off.data(), (size_t)n_lines + 1);
+    up(D.ln_kf, p->line_edge_kf, n_le);
+    up(D.ln_lm, p->line_edge_lm, n_le);
+    up(D.ln_obs, p->line_edge_obs, (size_t)n_le * 4);
+    up(D.ln_info, p->line_edge_inv_sigma_sq, n_le);
+    up(D.cta_ranges, ranges.data(), (size_t)G + 1);
+    up(b->d_T_in, p->kf_pose_cw, (size_t)n_kf * 16);
+    up(b->d_pts_in, p->pt_pos_w, (size_t)n_pts * 3);
+    up(b->d_lines_in, p->line_plucker, (size_t)n_lines * 6);
     if (up_err == cudaSuccess) up_err = cudaStreamSynchronize(ctx->stream);
     if (up_err != cudaSuccess) {
         set_error("local BA: upload failed: %s", cudaGetErrorString(up_err));
         plp_ba_destroy(b);
         return PLP_ERR_CUDA;
     }
-    b->d_stop = (double *)(d + o_stop);
-    BaDev &D = b->dev;
-    memset(&D, 0, sizeof(D));
+    if (!p->n_plane_edges) D.pt_plane = nullptr;
     D.fx = p->fx;
     D.fy = p->fy;
     D.cx = p->cx;
@@ -339,57 +367,6 @@ plp_status plp_ba_create(plp_ctx *ctx, const plp_ba_problem *p, const plp_ba_cfg
     D.world = world;
     D.large = large ? 1 : 0;
     D.phase_init_grid = 64;
-    D.dense = (double *)(d + o_dense);
-    D.kf_hidx = (int *)(d + o_hidx);
-    D.poses[0] = (se3::Pose *)(d + o_pose0);
-    D.poses[1] = (se3::Pose *)(d + o_pose1);
-    D.pert_pose = (se3::Pose *)(d + o_pert);
-    D.pair_bi = (int *)(d + o_pbi);
-    D.pair_bj = (int *)(d + o_pbj);
-    D.pts[0] = (double *)(d + o_pts0);
-    D.pts[1] = (double *)(d + o_pts1);
-    D.lines[0] = (double *)(d + o_ln0);
-    D.lines[1] = (double *)(d + o_ln1);
-    D.pt_off = (int *)(d + o_ptoff);
-    D.pt_kf = (int *)(d + o_ptkf);
-    D.pt_lm = (int *)(d + o_ptlm);
-    D.pt_obs = (float *)(d + o_ptobs);
-    D.pt_info = (float *)(d + o_ptinfo);
-    D.pt_level = d + o_ptlvl;
-    D.pt_outlier = d + o_ptout;
-    D.pt_chi2 = (double *)(d + o_ptchi);
-    D.pt_W = (double *)(d + o_ptW);
-    D.pt_Dinv = (double *)(d + o_ptD);
-    D.pt_bl = (double *)(d + o_ptbl);
-    D.pt_active = d + o_ptact;
-    D.pt_plane = p->n_plane_edges ? (int *)(d + o_ptplane) : nullptr;
-    D.pl_fn = (double *)(d + o_plfn);
-    D.pl_err = (double *)(d + o_plerr);
-    D.ln_off = (int *)(d + o_lnoff);
-    D.ln_kf = (int *)(d + o_lnkf);
-    D.ln_lm = (int *)(d + o_lnlm);
-    D.ln_obs = (float *)(d + o_lnobs);
-    D.ln_info = (float *)(d + o_lninfo);
-    D.ln_level = d + o_lnlvl;
-    D.ln_outlier = d + o_lnout;
-    D.ln_chi2 = (double *)(d + o_lnchi);
-    D.ln_W = (double *)(d + o_lnW);
-    D.ln_Dinv = (double *)(d + o_lnD);
-    D.ln_bl = (double *)(d + o_lnbl);
-    D.ln_active = d + o_lnact;
-    D.cta_ranges = (int *)(d + o_ranges);
-    D.partial = (double *)(d + o_partial);
-    D.packed = (double *)(d + o_packed);
-    D.dp = (double *)(d + o_dp);
-    D.trial_partial = (double *)(d + o_tp);
-    D.trial_sum = (double *)(d + o_ts);
-    D.state = (BaState *)(d + o_state);
-    b->d_T_in = (double *)(d + o_Tin);
-    b->d_pts_in = (double *)(d + o_ptsin);
-    b->d_lines_in = (double *)(d + o_lnin);
-    b->d_T_out = (double *)(d + o_Tout);
-    b->d_pts_out = (double *)(d + o_ptsout);
-    b->d_lines_out = (double *)(d + o_lnout2);
     *out = b;
     return PLP_OK;
 }

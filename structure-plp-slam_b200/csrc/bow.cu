@@ -223,16 +223,19 @@ plp_status plp_bow_transform(plp_bow_vocab *v, const uint8_t *desc, int n, int l
     PLP_REQUIRE(desc && word_id_out && node_id_out && weight_out, "null pointer");
     plp_ctx *ctx = v->ctx;
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
-    const size_t o_d = pk.add(desc, (size_t)n * 32);
-    const size_t o_w = pk.reserve((size_t)n * 4), o_n = pk.reserve((size_t)n * 4), o_f = pk.reserve((size_t)n * 4);
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    PLP_TRY(launch_transform(v, d + o_d, n, levelsup, Packer::at<int32_t>(d, o_w), Packer::at<int32_t>(d, o_n),
-                             Packer::at<float>(d, o_f)));
-    PLP_CUDA_TRY(cudaMemcpyAsync(word_id_out, d + o_w, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(node_id_out, d + o_n, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(weight_out, d + o_f, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    Layout lay;
+    const uint8_t *dd;
+    int32_t *dw, *dn;
+    float *df;
+    lay.in(dd, desc, (size_t)n * 32);
+    lay.out(dw, n);
+    lay.out(dn, n);
+    lay.out(df, n);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_TRY(launch_transform(v, dd, n, levelsup, dw, dn, df));
+    PLP_CUDA_TRY(cudaMemcpyAsync(word_id_out, dw, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(node_id_out, dn, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(weight_out, df, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return PLP_OK;
 }
@@ -241,12 +244,15 @@ plp_status plp_match_bow_tree(plp_ctx *ctx, plp_bow_pair *pairs, int num_pairs, 
     PLP_REQUIRE(ctx && num_pairs >= 0, "ctx / num_pairs");
     if (num_pairs == 0) return PLP_OK;
     PLP_REQUIRE(pairs, "pairs");
-    struct SideOff {
-        size_t desc, angle, valid, idx;
+    struct Side {
         std::vector<uint32_t> flat;  // validated copy of fv.indices
+        const uint8_t *desc;
+        const float *angle;
+        const uint8_t *valid;
+        const uint32_t *idx;
     };
-    std::map<const plp_bow_side *, SideOff> sides;
-    Packer pk;
+    std::map<const plp_bow_side *, Side> sides;
+    Layout lay;
     // validate + pack every distinct side once
     for (int p = 0; p < num_pairs; ++p) {
         pairs[p].num_matches = 0;
@@ -257,7 +263,7 @@ plp_status plp_match_bow_tree(plp_ctx *ctx, plp_bow_pair *pairs, int num_pairs, 
             PLP_REQUIRE(s->n == 0 || s->desc, "side descriptors");
             PLP_REQUIRE(s->fv.num_nodes == 0 || (s->fv.node_ids && s->fv.offsets && s->fv.indices), "feature vector");
             PLP_REQUIRE(!check_orientation || s->n == 0 || s->angle, "angles required for the orientation check");
-            SideOff so;
+            Side so;
             const int total = s->fv.num_nodes ? s->fv.offsets[s->fv.num_nodes] : 0;
             std::vector<uint8_t> seen((size_t)s->n, 0);
             for (int a = 0; a < s->fv.num_nodes; ++a) {
@@ -275,28 +281,28 @@ plp_status plp_match_bow_tree(plp_ctx *ctx, plp_bow_pair *pairs, int num_pairs, 
     }
     for (auto &kv : sides) {
         const plp_bow_side *s = kv.first;
-        SideOff &so = kv.second;
+        Side &so = kv.second;
         const size_t n = (size_t)s->n;
-        so.desc = pk.add(n ? s->desc : nullptr, n * 32);
-        so.angle = pk.add(n ? s->angle : nullptr, n * 4);
-        so.valid = pk.add(n ? s->valid : nullptr, n);
-        so.idx = pk.add(so.flat.empty() ? nullptr : so.flat.data(), so.flat.size() * 4);
+        lay.in(so.desc, s->desc, n * 32);
+        lay.in(so.angle, s->angle, n);
+        lay.in(so.valid, s->valid, n);
+        lay.in(so.idx, so.flat.data(), so.flat.size());
     }
     // merge-join of the two ascending feature vectors per pair (bow_tree.cc:60-150): the shared nodes
-    struct PairOff {
+    struct Shared {
         std::vector<int32_t> nb1, ne1, nb2, ne2;
-        size_t o_nb1, o_ne1, o_nb2, o_ne2, o_claimed, o_choice, o_m21, o_m12, o_num;
     };
-    std::vector<PairOff> po(num_pairs);
+    std::vector<Shared> sh(num_pairs);
+    std::vector<BowJob> jobs(num_pairs);
     for (int p = 0; p < num_pairs; ++p) {
         const plp_bow_feature_vector &f1 = pairs[p].side1->fv, &f2 = pairs[p].side2->fv;
         int a = 0, b = 0;
         while (a < f1.num_nodes && b < f2.num_nodes) {
             if (f1.node_ids[a] == f2.node_ids[b]) {
-                po[p].nb1.push_back(f1.offsets[a]);
-                po[p].ne1.push_back(f1.offsets[a + 1]);
-                po[p].nb2.push_back(f2.offsets[b]);
-                po[p].ne2.push_back(f2.offsets[b + 1]);
+                sh[p].nb1.push_back(f1.offsets[a]);
+                sh[p].ne1.push_back(f1.offsets[a + 1]);
+                sh[p].nb2.push_back(f2.offsets[b]);
+                sh[p].ne2.push_back(f2.offsets[b + 1]);
                 ++a;
                 ++b;
             } else if (f1.node_ids[a] < f2.node_ids[b]) {
@@ -305,74 +311,50 @@ plp_status plp_match_bow_tree(plp_ctx *ctx, plp_bow_pair *pairs, int num_pairs, 
                 ++b;
             }
         }
-        const size_t nn = po[p].nb1.size(), n1 = (size_t)pairs[p].side1->n, n2 = (size_t)pairs[p].side2->n;
-        po[p].o_nb1 = pk.add(nn ? po[p].nb1.data() : nullptr, nn * 4);
-        po[p].o_ne1 = pk.add(nn ? po[p].ne1.data() : nullptr, nn * 4);
-        po[p].o_nb2 = pk.add(nn ? po[p].nb2.data() : nullptr, nn * 4);
-        po[p].o_ne2 = pk.add(nn ? po[p].ne2.data() : nullptr, nn * 4);
-        po[p].o_claimed = pk.reserve(n2 + 1);
-        po[p].o_choice = pk.reserve(n1 * 4 + 4);
-    }
-    // all results in ONE contiguous region -> one D2H copy (a copy per pair and array costs more than the kernel)
-    const size_t o_out0 = pk.total;
-    for (int p = 0; p < num_pairs; ++p) {
-        const size_t n1 = (size_t)pairs[p].side1->n, n2 = (size_t)pairs[p].side2->n;
-        po[p].o_m21 = pk.reserve(n1 * 4 + 4);
-        po[p].o_m12 = pk.reserve(n2 * 4 + 4);
-        po[p].o_num = pk.reserve(4);
-    }
-    const size_t o_out1 = pk.total;
-    std::vector<BowJob> jobs(num_pairs);
-    const size_t o_jobs = pk.add(jobs.data(), sizeof(BowJob) * (size_t)num_pairs);
-    PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    void *dscratch = nullptr;
-    PLP_TRY(ctx_scratch(ctx, 0, pk.total ? pk.total : 256, &dscratch));
-    uint8_t *d = (uint8_t *)dscratch;
-    for (int p = 0; p < num_pairs; ++p) {
         BowJob &J = jobs[p];
-        memset(&J, 0, sizeof(J));
-        const SideOff &s1 = sides[pairs[p].side1], &s2 = sides[pairs[p].side2];
+        const Side &s1 = sides[pairs[p].side1], &s2 = sides[pairs[p].side2];
+        const size_t nn = sh[p].nb1.size();
         J.n1 = pairs[p].side1->n;
         J.n2 = pairs[p].side2->n;
-        J.num_nodes = (int)po[p].nb1.size();
-        J.desc1 = Packer::at<uint8_t>(d, s1.desc);
-        J.desc2 = Packer::at<uint8_t>(d, s2.desc);
-        J.angle1 = Packer::at<float>(d, s1.angle);
-        J.angle2 = Packer::at<float>(d, s2.angle);
-        J.valid1 = Packer::at<uint8_t>(d, s1.valid);
-        J.valid2 = Packer::at<uint8_t>(d, s2.valid);
-        J.idx1 = Packer::at<uint32_t>(d, s1.idx);
-        J.idx2 = Packer::at<uint32_t>(d, s2.idx);
-        J.nb1 = Packer::at<int32_t>(d, po[p].o_nb1);
-        J.ne1 = Packer::at<int32_t>(d, po[p].o_ne1);
-        J.nb2 = Packer::at<int32_t>(d, po[p].o_nb2);
-        J.ne2 = Packer::at<int32_t>(d, po[p].o_ne2);
-        J.claimed = Packer::at<uint8_t>(d, po[p].o_claimed);
-        J.choice = Packer::at<int32_t>(d, po[p].o_choice);
-        J.matched_2_of_1 = Packer::at<int32_t>(d, po[p].o_m21);
-        J.matched_1_of_2 = Packer::at<int32_t>(d, po[p].o_m12);
-        J.num_matches = Packer::at<uint32_t>(d, po[p].o_num);
+        J.num_nodes = (int)nn;
+        lay.alias(J.desc1, s1.desc);
+        lay.alias(J.desc2, s2.desc);
+        lay.alias(J.angle1, s1.angle);
+        lay.alias(J.angle2, s2.angle);
+        lay.alias(J.valid1, s1.valid);
+        lay.alias(J.valid2, s2.valid);
+        lay.alias(J.idx1, s1.idx);
+        lay.alias(J.idx2, s2.idx);
+        lay.in(J.nb1, sh[p].nb1.data(), nn);
+        lay.in(J.ne1, sh[p].ne1.data(), nn);
+        lay.in(J.nb2, sh[p].nb2.data(), nn);
+        lay.in(J.ne2, sh[p].ne2.data(), nn);
+        lay.out(J.claimed, (size_t)J.n2 + 1);
+        lay.out(J.choice, (size_t)J.n1 + 1);
     }
-    uint8_t *d2;
-    PLP_TRY(pk.upload(ctx, 0, &d2));
-    if (d2 != d) {
-        set_error("bow_tree: scratch buffer moved between sizing and upload");
-        return PLP_ERR_CUDA;
+    const BowJob *d_jobs;
+    lay.in(d_jobs, jobs.data(), num_pairs);
+    // all results in ONE contiguous region -> one D2H copy (a copy per pair and array costs more than the kernel)
+    for (BowJob &J : jobs) {
+        lay.out(J.matched_2_of_1, (size_t)J.n1 + 1);
+        lay.out(J.matched_1_of_2, (size_t)J.n2 + 1);
+        lay.out(J.num_matches, 1);
     }
-    PLP_LAUNCH(ctx, bow_match_kernel, num_pairs, kMatchThreads, 0, Packer::at<BowJob>(d, o_jobs), lowe_ratio,
-               check_orientation);
+    PLP_CUDA_TRY(cudaSetDevice(ctx->device));
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_LAUNCH(ctx, bow_match_kernel, num_pairs, kMatchThreads, 0, d_jobs, lowe_ratio, check_orientation);
     PLP_CHECK_LAUNCH();
-    void *hp = nullptr;
-    PLP_TRY(ctx_pinned(ctx, pk.total ? pk.total : 256, &hp));  // the staging buffer upload() just used
-    uint8_t *h = (uint8_t *)hp;
-    PLP_CUDA_TRY(cudaMemcpyAsync(h + o_out0, d + o_out0, o_out1 - o_out0, cudaMemcpyDeviceToHost, ctx->stream));
+    uint8_t *r0 = (uint8_t *)jobs[0].matched_2_of_1, *r1 = (uint8_t *)(jobs[num_pairs - 1].num_matches + 1);
+    PLP_CUDA_TRY(cudaMemcpyAsync(lay.staged(r0), r0, r1 - r0, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     std::vector<uint32_t> nums(num_pairs, 0);
     for (int p = 0; p < num_pairs; ++p) {
-        const size_t n1 = (size_t)pairs[p].side1->n, n2 = (size_t)pairs[p].side2->n;
-        if (pairs[p].matched_2_of_1_out && n1) memcpy(pairs[p].matched_2_of_1_out, h + po[p].o_m21, n1 * 4);
-        if (pairs[p].matched_1_of_2_out && n2) memcpy(pairs[p].matched_1_of_2_out, h + po[p].o_m12, n2 * 4);
-        memcpy(&nums[p], h + po[p].o_num, 4);
+        const BowJob &J = jobs[p];
+        if (pairs[p].matched_2_of_1_out && J.n1)
+            memcpy(pairs[p].matched_2_of_1_out, lay.staged(J.matched_2_of_1), (size_t)J.n1 * 4);
+        if (pairs[p].matched_1_of_2_out && J.n2)
+            memcpy(pairs[p].matched_1_of_2_out, lay.staged(J.matched_1_of_2), (size_t)J.n2 * 4);
+        nums[p] = *lay.staged(J.num_matches);
     }
     for (int p = 0; p < num_pairs; ++p) pairs[p].num_matches = nums[p];
     return PLP_OK;

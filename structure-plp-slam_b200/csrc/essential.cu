@@ -37,38 +37,33 @@ plp_status plp_essential_ransac(plp_ctx *ctx, const double *bearings_1, int n1, 
         return PLP_OK;
     }
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
+    Layout lay;
     const size_t M = (size_t)num_matches, K = (size_t)num_iter;
-    const size_t o_b1 = pk.add(bearings_1, (size_t)n1 * 24), o_b2 = pk.add(bearings_2, (size_t)n2 * 24);
-    const size_t o_m = pk.add(matches_12, M * 8), o_s = pk.add(samples, K * 32);
-    const size_t o_E = pk.reserve(K * 72), o_sc = pk.reserve(K * 4), o_in = pk.reserve(K * M), o_res = pk.reserve(K * M * 8);
-    const size_t o_bi = pk.reserve(M), o_bE = pk.reserve(72), o_bs = pk.reserve(8), o_v = pk.reserve(4);
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
     EssJob J;
-    J.b1 = Packer::at<double>(d, o_b1);
-    J.b2 = Packer::at<double>(d, o_b2);
-    J.matches = Packer::at<int32_t>(d, o_m);
-    J.samples = Packer::at<int32_t>(d, o_s);
+    lay.in(J.b1, bearings_1, (size_t)n1 * 3);
+    lay.in(J.b2, bearings_2, (size_t)n2 * 3);
+    lay.in(J.matches, matches_12, M * 2);
+    lay.in(J.samples, samples, K * 8);
+    lay.out(J.E, K * 9);
+    lay.out(J.score, K);
+    lay.out(J.inlier, K * M);
+    lay.out(J.res, K * M * 2);
+    lay.out(J.best_inlier, M);
+    lay.out(J.best_E, 9);
+    lay.out(J.best_score, 1);
+    lay.out(J.valid, 1);
     J.num_matches = num_matches;
     J.num_iter = num_iter;
     J.recompute = recompute;
-    J.E = Packer::at<double>(d, o_E);
-    J.score = Packer::at<float>(d, o_sc);
-    J.inlier = Packer::at<uint8_t>(d, o_in);
-    J.res = Packer::at<float>(d, o_res);
-    J.best_inlier = Packer::at<uint8_t>(d, o_bi);
-    J.best_E = Packer::at<double>(d, o_bE);
-    J.best_score = Packer::at<double>(d, o_bs);
-    J.valid = Packer::at<int32_t>(d, o_v);
+    PLP_TRY(lay.upload(ctx, 0));
     PLP_LAUNCH(ctx, essential_hypothesis_kernel, num_iter, kEssThreads, 0, J);
     PLP_CHECK_LAUNCH();
     PLP_LAUNCH(ctx, essential_select_kernel, 1, kEssThreads, 0, J);
     PLP_CHECK_LAUNCH();
-    PLP_CUDA_TRY(cudaMemcpyAsync(is_inlier_out, d + o_bi, M, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(best_E_21_out, d + o_bE, 72, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(best_score_out, d + o_bs, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(solution_is_valid_out, d + o_v, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(is_inlier_out, J.best_inlier, M, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(best_E_21_out, J.best_E, 72, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(best_score_out, J.best_score, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(solution_is_valid_out, J.valid, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return PLP_OK;
 }

@@ -115,32 +115,16 @@ static plp_status fill_params(FuseParams &P, const plp_camera *cam, const plp_gr
     return PLP_OK;
 }
 
-struct LmOffsets {
-    size_t pos, normal, min_d, max_d, max_raw, desc, valid;
-};
-
-static void pack_landmarks(Packer &pk, const plp_fuse_landmarks *lms, int doubles_per_lm, LmOffsets &o) {
-    const size_t m = (size_t)lms->m;
-    o.pos = pk.add(lms->pos_w, m * doubles_per_lm * 8);
-    o.normal = pk.add(lms->obs_mean_normal, m * 3 * 8);
-    o.min_d = pk.add(lms->min_valid_dist, m * 4);
-    o.max_d = pk.add(lms->max_valid_dist, m * 4);
-    o.max_raw = pk.add(lms->max_valid_dist_raw, m * 4);
-    o.desc = pk.add(lms->desc, m * 32);
-    o.valid = pk.add(lms->valid, m);
-}
-
-static FuseLandmarks bind_landmarks(uint8_t *d, const LmOffsets &o, int m) {
-    FuseLandmarks L;
-    L.m = m;
-    L.pos_w = Packer::at<double>(d, o.pos);
-    L.normal = Packer::at<double>(d, o.normal);
-    L.min_d = Packer::at<float>(d, o.min_d);
-    L.max_d = Packer::at<float>(d, o.max_d);
-    L.max_raw = Packer::at<float>(d, o.max_raw);
-    L.desc = Packer::at<uint8_t>(d, o.desc);
-    L.valid = Packer::at<uint8_t>(d, o.valid);
-    return L;
+static void add_landmarks(Layout &lay, const plp_fuse_landmarks &lms, int doubles_per_lm, FuseLandmarks &L) {
+    const size_t m = (size_t)lms.m;
+    L.m = lms.m;
+    lay.in(L.pos_w, lms.pos_w, m * doubles_per_lm);
+    lay.in(L.normal, lms.obs_mean_normal, m * 3);
+    lay.in(L.min_d, lms.min_valid_dist, m);
+    lay.in(L.max_d, lms.max_valid_dist, m);
+    lay.in(L.max_raw, lms.max_valid_dist_raw, m);
+    lay.in(L.desc, lms.desc, m * 32);
+    lay.in(L.valid, lms.valid, m);
 }
 
 // landmarks per CTA so that (chunks x targets) fills the GPU about twice
@@ -196,62 +180,42 @@ plp_status plp_fuse_search_points(plp_ctx *ctx, const plp_fuse_target_points *ta
     FuseParams P;
     PLP_TRY(fill_params(P, cam, grid, scale_factors, inv_level_sigma_sq, num_levels, log_scale_factor, margin, mode));
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
-    LmOffsets lo;
-    pack_landmarks(pk, lms, 3, lo);
-    struct TOff {
-        size_t x, y, xr, oct, desc, skip;
-    };
-    std::vector<TOff> toff(num_targets);
+    Layout lay;
+    FuseLandmarks L;
+    add_landmarks(lay, *lms, 3, L);
+    std::vector<FusePointTarget> dev_targets(num_targets);
     for (int t = 0; t < num_targets; ++t) {
         const plp_frame_points &f = targets[t].pts;
         const size_t n = (size_t)f.n;
-        toff[t].x = pk.add(n ? f.x : nullptr, n * 4);
-        toff[t].y = pk.add(n ? f.y : nullptr, n * 4);
-        toff[t].xr = pk.add(n ? f.x_right : nullptr, n * 4);
-        toff[t].oct = pk.add(n ? f.octave : nullptr, n * 4);
-        toff[t].desc = pk.add(n ? f.desc : nullptr, n * 32);
-        toff[t].skip = pk.add(targets[t].skip, (size_t)m);
-    }
-    std::vector<FusePointTarget> dev_targets(num_targets);
-    const size_t o_targets = pk.add(dev_targets.data(), sizeof(FusePointTarget) * (size_t)num_targets);
-    const size_t o_idx = pk.reserve((size_t)num_targets * m * 4), o_dist = pk.reserve((size_t)num_targets * m * 2);
-    // device addresses are known once the scratch buffer is sized: size it first, then fill the target table in place
-    void *dscratch = nullptr;
-    PLP_TRY(ctx_scratch(ctx, 0, pk.total ? pk.total : 256, &dscratch));
-    uint8_t *d = (uint8_t *)dscratch;
-    for (int t = 0; t < num_targets; ++t) {
         FusePointTarget &T = dev_targets[t];
-        memset(&T, 0, sizeof(T));
-        T.n = targets[t].pts.n;
-        T.x = Packer::at<float>(d, toff[t].x);
-        T.y = Packer::at<float>(d, toff[t].y);
-        T.xr = Packer::at<float>(d, toff[t].xr);
-        T.octave = Packer::at<int32_t>(d, toff[t].oct);
-        T.desc = Packer::at<uint8_t>(d, toff[t].desc);
-        T.skip = Packer::at<uint8_t>(d, toff[t].skip);
+        T.n = f.n;
+        lay.in(T.x, f.x, n);
+        lay.in(T.y, f.y, n);
+        lay.in(T.xr, f.x_right, n);
+        lay.in(T.octave, f.octave, n);
+        lay.in(T.desc, f.desc, n * 32);
+        lay.in(T.skip, targets[t].skip, m);
         memcpy(T.R, targets[t].rot_cw, sizeof(T.R));
         memcpy(T.t, targets[t].trans_cw, sizeof(T.t));
         memcpy(T.c, targets[t].cam_center, sizeof(T.c));
     }
-    uint8_t *d2;
-    PLP_TRY(pk.upload(ctx, 0, &d2));
-    if (d2 != d) {
-        set_error("fuse: scratch buffer moved between sizing and upload");
-        return PLP_ERR_CUDA;
-    }
-    const FuseLandmarks L = bind_landmarks(d, lo, m);
+    const FusePointTarget *d_targets;
+    int32_t *d_idx;
+    uint16_t *d_dist;
+    lay.in(d_targets, dev_targets.data(), num_targets);
+    lay.out(d_idx, (size_t)num_targets * m);
+    lay.out(d_dist, (size_t)num_targets * m);
+    PLP_TRY(lay.upload(ctx, 0));
     const int cap = max_n < 64 ? 64 : ((max_n + 63) / 64) * 64;
     const size_t smem = fuse_point_smem_bytes(cap, grid->num_cols * grid->num_rows);
     PLP_SMEM_OPTIN(fuse_points_kernel, smem);
     const int chunk = chunk_size(ctx, m, num_targets);
     dim3 g(div_up(m, chunk), num_targets);
-    PLP_LAUNCH(ctx, fuse_points_kernel, g, kThreads, smem, Packer::at<FusePointTarget>(d, o_targets), L, P, cap, chunk,
-               Packer::at<int32_t>(d, o_idx), Packer::at<uint16_t>(d, o_dist));
+    PLP_LAUNCH(ctx, fuse_points_kernel, g, kThreads, smem, d_targets, L, P, cap, chunk, d_idx, d_dist);
     PLP_CHECK_LAUNCH();
-    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, d + o_idx, (size_t)num_targets * m * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, d_idx, (size_t)num_targets * m * 4, cudaMemcpyDeviceToHost, ctx->stream));
     if (best_dist_out)
-        PLP_CUDA_TRY(cudaMemcpyAsync(best_dist_out, d + o_dist, (size_t)num_targets * m * 2, cudaMemcpyDeviceToHost,
+        PLP_CUDA_TRY(cudaMemcpyAsync(best_dist_out, d_dist, (size_t)num_targets * m * 2, cudaMemcpyDeviceToHost,
                                      ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return PLP_OK;
@@ -284,65 +248,45 @@ plp_status plp_fuse_search_lines(plp_ctx *ctx, const plp_fuse_target_lines *targ
     PLP_TRY(fill_params(P, cam, nullptr, scale_factors_lsd, inv_level_sigma_sq_lsd, num_levels_lsd, log_scale_factor_lsd,
                         margin, PLP_FUSE_REPLACE));
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
-    LmOffsets lo;
+    Layout lay;
+    FuseLandmarks L;
     plp_fuse_landmarks lms_no_normal = *lms;
     lms_no_normal.obs_mean_normal = nullptr;
-    pack_landmarks(pk, &lms_no_normal, 6, lo);
-    struct TOff {
-        size_t sx, sy, ex, ey, oct, desc, skip;
-    };
-    std::vector<TOff> toff(num_targets);
+    add_landmarks(lay, lms_no_normal, 6, L);
+    std::vector<FuseLineTarget> dev_targets(num_targets);
     for (int t = 0; t < num_targets; ++t) {
         const plp_frame_lines &f = targets[t].lines;
         const size_t n = (size_t)f.n;
-        toff[t].sx = pk.add(n ? f.sx : nullptr, n * 4);
-        toff[t].sy = pk.add(n ? f.sy : nullptr, n * 4);
-        toff[t].ex = pk.add(n ? f.ex : nullptr, n * 4);
-        toff[t].ey = pk.add(n ? f.ey : nullptr, n * 4);
-        toff[t].oct = pk.add(n ? f.octave : nullptr, n * 4);
-        toff[t].desc = pk.add(n ? f.desc : nullptr, n * 32);
-        toff[t].skip = pk.add(targets[t].skip, (size_t)m);
-    }
-    std::vector<FuseLineTarget> dev_targets(num_targets);
-    const size_t o_targets = pk.add(dev_targets.data(), sizeof(FuseLineTarget) * (size_t)num_targets);
-    const size_t o_idx = pk.reserve((size_t)num_targets * m * 4), o_dist = pk.reserve((size_t)num_targets * m * 2);
-    void *dscratch = nullptr;
-    PLP_TRY(ctx_scratch(ctx, 0, pk.total ? pk.total : 256, &dscratch));
-    uint8_t *d = (uint8_t *)dscratch;
-    for (int t = 0; t < num_targets; ++t) {
         FuseLineTarget &T = dev_targets[t];
-        memset(&T, 0, sizeof(T));
-        T.n = targets[t].lines.n;
-        T.sx = Packer::at<float>(d, toff[t].sx);
-        T.sy = Packer::at<float>(d, toff[t].sy);
-        T.ex = Packer::at<float>(d, toff[t].ex);
-        T.ey = Packer::at<float>(d, toff[t].ey);
-        T.octave = Packer::at<int32_t>(d, toff[t].oct);
-        T.desc = Packer::at<uint8_t>(d, toff[t].desc);
-        T.skip = Packer::at<uint8_t>(d, toff[t].skip);
+        T.n = f.n;
+        lay.in(T.sx, f.sx, n);
+        lay.in(T.sy, f.sy, n);
+        lay.in(T.ex, f.ex, n);
+        lay.in(T.ey, f.ey, n);
+        lay.in(T.octave, f.octave, n);
+        lay.in(T.desc, f.desc, n * 32);
+        lay.in(T.skip, targets[t].skip, m);
         memcpy(T.R, targets[t].rot_cw, sizeof(T.R));
         memcpy(T.t, targets[t].trans_cw, sizeof(T.t));
         memcpy(T.c, targets[t].cam_center, sizeof(T.c));
     }
-    uint8_t *d2;
-    PLP_TRY(pk.upload(ctx, 0, &d2));
-    if (d2 != d) {
-        set_error("fuse: scratch buffer moved between sizing and upload");
-        return PLP_ERR_CUDA;
-    }
-    const FuseLandmarks L = bind_landmarks(d, lo, m);
+    const FuseLineTarget *d_targets;
+    int32_t *d_idx;
+    uint16_t *d_dist;
+    lay.in(d_targets, dev_targets.data(), num_targets);
+    lay.out(d_idx, (size_t)num_targets * m);
+    lay.out(d_dist, (size_t)num_targets * m);
+    PLP_TRY(lay.upload(ctx, 0));
     const int cap = max_n < 64 ? 64 : ((max_n + 63) / 64) * 64;
     const size_t smem = (size_t)cap * (32 + 5 * 4);
     PLP_SMEM_OPTIN(fuse_lines_kernel, smem);
     const int chunk = chunk_size(ctx, m, num_targets);
     dim3 g(div_up(m, chunk), num_targets);
-    PLP_LAUNCH(ctx, fuse_lines_kernel, g, kThreads, smem, Packer::at<FuseLineTarget>(d, o_targets), L, P, cap, chunk,
-               Packer::at<int32_t>(d, o_idx), Packer::at<uint16_t>(d, o_dist));
+    PLP_LAUNCH(ctx, fuse_lines_kernel, g, kThreads, smem, d_targets, L, P, cap, chunk, d_idx, d_dist);
     PLP_CHECK_LAUNCH();
-    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, d + o_idx, (size_t)num_targets * m * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, d_idx, (size_t)num_targets * m * 4, cudaMemcpyDeviceToHost, ctx->stream));
     if (best_dist_out)
-        PLP_CUDA_TRY(cudaMemcpyAsync(best_dist_out, d + o_dist, (size_t)num_targets * m * 2, cudaMemcpyDeviceToHost,
+        PLP_CUDA_TRY(cudaMemcpyAsync(best_dist_out, d_dist, (size_t)num_targets * m * 2, cudaMemcpyDeviceToHost,
                                      ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return PLP_OK;

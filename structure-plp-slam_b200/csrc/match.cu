@@ -701,16 +701,17 @@ plp_status plp_hamming_matrix(plp_ctx *ctx, const uint8_t *a, int na, const uint
     if (na == 0 || nb == 0) return PLP_OK;
     PLP_REQUIRE(a && b && dist_out, "null pointer");
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
-    const size_t oa = pk.add(a, (size_t)na * 32), ob = pk.add(b, (size_t)nb * 32);
-    const size_t oo = pk.reserve((size_t)na * nb * 2);
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
+    Layout lay;
+    const uint8_t *da, *db;
+    uint16_t *dist;
+    lay.in(da, a, (size_t)na * 32);
+    lay.in(db, b, (size_t)nb * 32);
+    lay.out(dist, (size_t)na * nb);
+    PLP_TRY(lay.upload(ctx, 0));
     dim3 grid(div_up(nb, 32), div_up(na, 32)), block(32, 8);
-    PLP_LAUNCH(ctx, hamming_matrix_kernel, grid, block, 0, Packer::at<uint8_t>(d, oa), na, Packer::at<uint8_t>(d, ob), nb,
-               Packer::at<uint16_t>(d, oo));
+    PLP_LAUNCH(ctx, hamming_matrix_kernel, grid, block, 0, da, na, db, nb, dist);
     PLP_CHECK_LAUNCH();
-    PLP_CUDA_TRY(cudaMemcpyAsync(dist_out, d + oo, (size_t)na * nb * 2, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(dist_out, dist, (size_t)na * nb * 2, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return PLP_OK;
 }
@@ -728,41 +729,34 @@ plp_status plp_hamming_nn(plp_ctx *ctx, const uint8_t *query, int nq, const uint
         return PLP_OK;
     }
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
-    const size_t oq = pk.add(query, (size_t)nq * 32), ot = pk.add(train, (size_t)nt * 32);
-    const size_t oi = pk.reserve((size_t)nq * 4), od = pk.reserve((size_t)nq * 2);
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    PLP_LAUNCH(ctx, hamming_nn_kernel, div_up(nq * 32, 256), 256, 0, Packer::at<uint8_t>(d, oq), nq,
-               Packer::at<uint8_t>(d, ot), nt, Packer::at<int32_t>(d, oi), Packer::at<uint16_t>(d, od));
+    Layout lay;
+    const uint8_t *dq, *dt;
+    int32_t *di;
+    uint16_t *dd;
+    lay.in(dq, query, (size_t)nq * 32);
+    lay.in(dt, train, (size_t)nt * 32);
+    lay.out(di, nq);
+    lay.out(dd, nq);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_LAUNCH(ctx, hamming_nn_kernel, div_up(nq * 32, 256), 256, 0, dq, nq, dt, nt, di, dd);
     PLP_CHECK_LAUNCH();
-    PLP_CUDA_TRY(cudaMemcpyAsync(nn_idx, d + oi, (size_t)nq * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(nn_dist, d + od, (size_t)nq * 2, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(nn_idx, di, (size_t)nq * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(nn_dist, dd, (size_t)nq * 2, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return PLP_OK;
 }
 
-static plp_status pack_frame_points(Packer &pk, const plp_frame_points *f, PointMatchJob &J, size_t off[7]) {
-    const size_t n = (size_t)f->n;
-    off[0] = pk.add(f->x, n * 4);
-    off[1] = pk.add(f->y, n * 4);
-    off[2] = pk.add(f->octave, n * 4);
-    off[3] = pk.add(f->angle, n * 4);
-    off[4] = pk.add(f->x_right, n * 4);
-    off[5] = pk.add(f->desc, n * 32);
-    off[6] = pk.add(f->claimed, n);
-    J.n = f->n;
-    return PLP_OK;
-}
-
-static void bind_frame_points(uint8_t *d, const size_t off[7], PointMatchJob &J) {
-    J.x = Packer::at<float>(d, off[0]);
-    J.y = Packer::at<float>(d, off[1]);
-    J.octave = Packer::at<int32_t>(d, off[2]);
-    J.angle = Packer::at<float>(d, off[3]);
-    J.x_right = Packer::at<float>(d, off[4]);
-    J.desc = Packer::at<uint8_t>(d, off[5]);
-    J.claimed = Packer::at<uint8_t>(d, off[6]);
+// the frame's keypoints as the candidate side of a window-matcher job
+static void add_frame_points(Layout &lay, const plp_frame_points &f, PointMatchJob &J) {
+    const size_t n = (size_t)f.n;
+    J.n = f.n;
+    lay.in(J.x, f.x, n);
+    lay.in(J.y, f.y, n);
+    lay.in(J.octave, f.octave, n);
+    lay.in(J.angle, f.angle, n);
+    lay.in(J.x_right, f.x_right, n);
+    lay.in(J.desc, f.desc, n * 32);
+    lay.in(J.claimed, f.claimed, n);
 }
 
 plp_status plp_match_frame_and_landmarks(plp_ctx *ctx, const plp_frame_points *frm, const plp_grid *grid,
@@ -791,38 +785,31 @@ plp_status plp_match_frame_and_landmarks(plp_ctx *ctx, const plp_frame_points *f
         qmin[i] = lvl - 1;
         qmax[i] = lvl;
     }
-    Packer pk;
+    Layout lay;
     PointMatchJob J;
     memset(&J, 0, sizeof(J));
-    size_t fo[7];
-    pack_frame_points(pk, frm, J, fo);
-    const size_t o_qx = pk.add(q->reproj_x, (size_t)m * 4), o_qy = pk.add(q->reproj_y, (size_t)m * 4);
-    const size_t o_qxr = pk.add(q->x_right, (size_t)m * 4);
-    const size_t o_r = pk.add(radius.data(), (size_t)m * 4);
-    const size_t o_mn = pk.add(qmin.data(), (size_t)m * 4), o_mx = pk.add(qmax.data(), (size_t)m * 4);
-    const size_t o_qd = pk.add(q->desc, (size_t)m * 32), o_qv = pk.add(q->valid, (size_t)m);
-    const size_t o_choice = pk.reserve((size_t)m * 4), o_best = pk.reserve((size_t)m * 4), o_num = pk.reserve(4);
-    const size_t o_job = pk.reserve(sizeof(PointMatchJob));
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    bind_frame_points(d, fo, J);
+    plp_frame_points f = *frm;
+    f.angle = nullptr;  // no orientation check here: the matcher never reads the frame's angles
+    add_frame_points(lay, f, J);
     J.m = m;
-    J.qx = Packer::at<float>(d, o_qx);
-    J.qy = Packer::at<float>(d, o_qy);
-    J.qxr = Packer::at<float>(d, o_qxr);
-    J.qradius = Packer::at<float>(d, o_r);
-    J.qmin = Packer::at<int32_t>(d, o_mn);
-    J.qmax = Packer::at<int32_t>(d, o_mx);
-    J.qdesc = Packer::at<uint8_t>(d, o_qd);
-    J.qvalid = Packer::at<uint8_t>(d, o_qv);
-    J.choice = Packer::at<int32_t>(d, o_choice);
-    J.best_idx_out = Packer::at<int32_t>(d, o_best);
-    J.num_matches = Packer::at<uint32_t>(d, o_num);
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_job, &J, sizeof(J), cudaMemcpyHostToDevice, ctx->stream));
-    PLP_TRY(launch_point_match(ctx, Packer::at<PointMatchJob>(d, o_job), 1, frm->n, *grid, 1, lowe_ratio, 0));
+    lay.in(J.qx, q->reproj_x, m);
+    lay.in(J.qy, q->reproj_y, m);
+    lay.in(J.qxr, q->x_right, m);
+    lay.in(J.qradius, radius.data(), m);
+    lay.in(J.qmin, qmin.data(), m);
+    lay.in(J.qmax, qmax.data(), m);
+    lay.in(J.qdesc, q->desc, (size_t)m * 32);
+    lay.in(J.qvalid, q->valid, m);
+    const PointMatchJob *d_job;
+    lay.in(d_job, &J, 1);
+    lay.out(J.choice, m);
+    lay.out(J.best_idx_out, m);
+    lay.out(J.num_matches, 1);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_TRY(launch_point_match(ctx, d_job, 1, frm->n, *grid, 1, lowe_ratio, 0));
     uint32_t num = 0;
-    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, d + o_best, (size_t)m * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(&num, d + o_num, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, J.best_idx_out, (size_t)m * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(&num, J.num_matches, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (num_matches_out) *num_matches_out = num;
     return PLP_OK;
@@ -846,91 +833,71 @@ plp_status plp_match_current_and_last_frames(plp_ctx *ctx, const plp_frame_point
     for (int i = 0; i < last->n; ++i) PLP_REQUIRE(last->octave[i] >= 0 && last->octave[i] < num_levels, "octave range");
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
     const int m = last->n, n = curr->n;
-    Packer pk;
+    Layout lay;
     PointMatchJob J;
     memset(&J, 0, sizeof(J));
     ProjectJob P;
     memset(&P, 0, sizeof(P));
-    size_t fo[7];
-    pack_frame_points(pk, curr, J, fo);
-    const size_t o_pw = pk.add(last->pos_w, (size_t)m * 24), o_oct = pk.add(last->octave, (size_t)m * 4);
-    const size_t o_ang = pk.add(last->angle, (size_t)m * 4), o_qd = pk.add(last->desc, (size_t)m * 32);
-    const size_t o_val = pk.add(last->valid, (size_t)m);
-    const size_t o_sf = pk.add(scale_factors, (size_t)num_levels * 4);
-    const size_t o_qx = pk.reserve((size_t)m * 4), o_qy = pk.reserve((size_t)m * 4), o_qxr = pk.reserve((size_t)m * 4);
-    const size_t o_r = pk.reserve((size_t)m * 4), o_mn = pk.reserve((size_t)m * 4), o_mx = pk.reserve((size_t)m * 4);
-    const size_t o_qv = pk.reserve((size_t)m);
-    const size_t o_choice = pk.reserve((size_t)m * 4), o_matched = pk.reserve((size_t)n * 4), o_num = pk.reserve(4);
-    const size_t o_job = pk.reserve(sizeof(PointMatchJob)), o_pjob = pk.reserve(sizeof(ProjectJob));
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    bind_frame_points(d, fo, J);
+    add_frame_points(lay, *curr, J);
     P.n_last = m;
-    P.pos_w = Packer::at<double>(d, o_pw);
-    P.octave = Packer::at<int32_t>(d, o_oct);
-    P.valid = Packer::at<uint8_t>(d, o_val);
+    lay.in(P.pos_w, last->pos_w, (size_t)m * 3);
+    lay.in(P.octave, last->octave, m);
+    lay.in(J.qangle, last->angle, m);
+    lay.in(J.qdesc, last->desc, (size_t)m * 32);
+    lay.in(P.valid, last->valid, m);
+    const float *d_sf;
+    lay.in(d_sf, scale_factors, num_levels);
     for (int r = 0; r < 3; ++r)
         for (int c = 0; c < 4; ++c) P.pose_cw[r * 4 + c] = pose_cw_curr[r * 4 + c];
     motion_assumption(*cam, pose_cw_curr, pose_cw_last, &P.assume_forward, &P.assume_backward);
-    P.qx = Packer::at<float>(d, o_qx);
-    P.qy = Packer::at<float>(d, o_qy);
-    P.qxr = Packer::at<float>(d, o_qxr);
-    P.qradius = Packer::at<float>(d, o_r);
-    P.qmin = Packer::at<int32_t>(d, o_mn);
-    P.qmax = Packer::at<int32_t>(d, o_mx);
-    P.qvalid = Packer::at<uint8_t>(d, o_qv);
     J.m = m;
-    J.qx = P.qx;
-    J.qy = P.qy;
-    J.qxr = P.qxr;
-    J.qradius = P.qradius;
-    J.qmin = P.qmin;
-    J.qmax = P.qmax;
-    J.qangle = Packer::at<float>(d, o_ang);
-    J.qdesc = Packer::at<uint8_t>(d, o_qd);
-    J.qvalid = P.qvalid;
-    J.choice = Packer::at<int32_t>(d, o_choice);
-    J.matched_out = Packer::at<int32_t>(d, o_matched);
-    J.num_matches = Packer::at<uint32_t>(d, o_num);
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_job, &J, sizeof(J), cudaMemcpyHostToDevice, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_pjob, &P, sizeof(P), cudaMemcpyHostToDevice, ctx->stream));
-    PLP_TRY(launch_project_points(ctx, Packer::at<ProjectJob>(d, o_pjob), 1, m, *cam, Packer::at<float>(d, o_sf),
-                                  num_levels, margin));
-    PLP_TRY(launch_point_match(ctx, Packer::at<PointMatchJob>(d, o_job), 1, n, *grid, 0, 0.0f, check_orientation));
+    const PointMatchJob *d_job;
+    const ProjectJob *d_pjob;
+    lay.in(d_job, &J, 1);
+    lay.in(d_pjob, &P, 1);
+    // the projection pre-pass writes the queries the matcher reads
+    lay.out(P.qx, m);
+    lay.out(P.qy, m);
+    lay.out(P.qxr, m);
+    lay.out(P.qradius, m);
+    lay.out(P.qmin, m);
+    lay.out(P.qmax, m);
+    lay.out(P.qvalid, m);
+    lay.alias(J.qx, P.qx);
+    lay.alias(J.qy, P.qy);
+    lay.alias(J.qxr, P.qxr);
+    lay.alias(J.qradius, P.qradius);
+    lay.alias(J.qmin, P.qmin);
+    lay.alias(J.qmax, P.qmax);
+    lay.alias(J.qvalid, P.qvalid);
+    lay.out(J.choice, m);
+    lay.out(J.matched_out, n);
+    lay.out(J.num_matches, 1);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_TRY(launch_project_points(ctx, d_pjob, 1, m, *cam, d_sf, num_levels, margin));
+    PLP_TRY(launch_point_match(ctx, d_job, 1, n, *grid, 0, 0.0f, check_orientation));
     uint32_t num = 0;
-    PLP_CUDA_TRY(cudaMemcpyAsync(matched_last_idx_out, d + o_matched, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(&num, d + o_num, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(matched_last_idx_out, J.matched_out, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(&num, J.num_matches, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (num_matches_out) *num_matches_out = num;
     return PLP_OK;
 }
 
-static void pack_frame_lines(Packer &pk, const plp_frame_lines *f, size_t off[11]) {
-    const size_t n = (size_t)f->n;
-    off[0] = pk.add(f->sx, n * 4);
-    off[1] = pk.add(f->sy, n * 4);
-    off[2] = pk.add(f->ex, n * 4);
-    off[3] = pk.add(f->ey, n * 4);
-    off[4] = pk.add(f->octave, n * 4);
-    off[5] = pk.add(f->ratio_level, n * 4);
-    off[6] = pk.add(f->x_right_sp, n * 4);
-    off[7] = pk.add(f->x_right_ep, n * 4);
-    off[8] = pk.add(f->desc, n * 32);
-    off[9] = pk.add(f->claimed, n);
-}
-
-static void bind_frame_lines(uint8_t *d, const size_t off[11], const plp_frame_lines *f, LineMatchJob &J) {
-    J.n = f->n;
-    J.sx = Packer::at<float>(d, off[0]);
-    J.sy = Packer::at<float>(d, off[1]);
-    J.ex = Packer::at<float>(d, off[2]);
-    J.ey = Packer::at<float>(d, off[3]);
-    J.octave = Packer::at<int32_t>(d, off[4]);
-    J.ratio_level = Packer::at<int32_t>(d, off[5]);
-    J.xr_sp = Packer::at<float>(d, off[6]);
-    J.xr_ep = Packer::at<float>(d, off[7]);
-    J.desc = Packer::at<uint8_t>(d, off[8]);
-    J.claimed = Packer::at<uint8_t>(d, off[9]);
+// the frame's keylines as the candidate side of a keyline-matcher job
+static void add_frame_lines(Layout &lay, const plp_frame_lines &f, LineMatchJob &J) {
+    const size_t n = (size_t)f.n;
+    J.n = f.n;
+    lay.in(J.sx, f.sx, n);
+    lay.in(J.sy, f.sy, n);
+    lay.in(J.ex, f.ex, n);
+    lay.in(J.ey, f.ey, n);
+    lay.in(J.octave, f.octave, n);
+    lay.in(J.ratio_level, f.ratio_level, n);
+    lay.in(J.xr_sp, f.x_right_sp, n);
+    lay.in(J.xr_ep, f.x_right_ep, n);
+    lay.in(J.desc, f.desc, n * 32);
+    lay.in(J.claimed, f.claimed, n);
 }
 
 plp_status plp_match_frame_and_landmarks_line(plp_ctx *ctx, const plp_frame_lines *frm, const float *scale_factors_lsd,
@@ -958,39 +925,30 @@ plp_status plp_match_frame_and_landmarks_line(plp_ctx *ctx, const plp_frame_line
         qmin[i] = lvl - 1;
         qmax[i] = lvl;
     }
-    Packer pk;
+    Layout lay;
     LineMatchJob J;
     memset(&J, 0, sizeof(J));
-    size_t fo[11];
-    pack_frame_lines(pk, frm, fo);
-    const size_t o1 = pk.add(q->sp_x, (size_t)m * 4), o2 = pk.add(q->sp_y, (size_t)m * 4);
-    const size_t o3 = pk.add(q->ep_x, (size_t)m * 4), o4 = pk.add(q->ep_y, (size_t)m * 4);
-    const size_t o_r = pk.add(radius.data(), (size_t)m * 4);
-    const size_t o_mn = pk.add(qmin.data(), (size_t)m * 4), o_mx = pk.add(qmax.data(), (size_t)m * 4);
-    const size_t o_qd = pk.add(q->desc, (size_t)m * 32), o_qv = pk.add(q->valid, (size_t)m);
-    const size_t o_choice = pk.reserve((size_t)m * 4), o_best = pk.reserve((size_t)m * 4), o_num = pk.reserve(4);
-    const size_t o_job = pk.reserve(sizeof(LineMatchJob));
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    bind_frame_lines(d, fo, frm, J);
+    add_frame_lines(lay, *frm, J);
     J.m = m;
-    J.q_spx = Packer::at<float>(d, o1);
-    J.q_spy = Packer::at<float>(d, o2);
-    J.q_epx = Packer::at<float>(d, o3);
-    J.q_epy = Packer::at<float>(d, o4);
-    J.qradius = Packer::at<float>(d, o_r);
-    J.qmin = Packer::at<int32_t>(d, o_mn);
-    J.qmax = Packer::at<int32_t>(d, o_mx);
-    J.qdesc = Packer::at<uint8_t>(d, o_qd);
-    J.qvalid = Packer::at<uint8_t>(d, o_qv);
-    J.choice = Packer::at<int32_t>(d, o_choice);
-    J.best_idx_out = Packer::at<int32_t>(d, o_best);
-    J.num_matches = Packer::at<uint32_t>(d, o_num);
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_job, &J, sizeof(J), cudaMemcpyHostToDevice, ctx->stream));
-    PLP_TRY(launch_line_match(ctx, Packer::at<LineMatchJob>(d, o_job), 1, 1, lowe_ratio, 0));
+    lay.in(J.q_spx, q->sp_x, m);
+    lay.in(J.q_spy, q->sp_y, m);
+    lay.in(J.q_epx, q->ep_x, m);
+    lay.in(J.q_epy, q->ep_y, m);
+    lay.in(J.qradius, radius.data(), m);
+    lay.in(J.qmin, qmin.data(), m);
+    lay.in(J.qmax, qmax.data(), m);
+    lay.in(J.qdesc, q->desc, (size_t)m * 32);
+    lay.in(J.qvalid, q->valid, m);
+    const LineMatchJob *d_job;
+    lay.in(d_job, &J, 1);
+    lay.out(J.choice, m);
+    lay.out(J.best_idx_out, m);
+    lay.out(J.num_matches, 1);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_TRY(launch_line_match(ctx, d_job, 1, 1, lowe_ratio, 0));
     uint32_t num = 0;
-    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, d + o_best, (size_t)m * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(&num, d + o_num, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, J.best_idx_out, (size_t)m * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(&num, J.num_matches, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (num_matches_out) *num_matches_out = num;
     return PLP_OK;
@@ -1016,66 +974,59 @@ plp_status plp_match_current_and_last_frames_line(plp_ctx *ctx, const plp_frame_
         PLP_REQUIRE(last->octave[i] >= 0 && last->octave[i] < num_levels_lsd, "octave range");
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
     const int m = last->n, n = curr->n;
-    Packer pk;
+    Layout lay;
     LineMatchJob J;
     memset(&J, 0, sizeof(J));
     ProjectJob P;
     memset(&P, 0, sizeof(P));
-    size_t fo[11];
-    pack_frame_lines(pk, curr, fo);
-    const size_t o_pw = pk.add(last->pos_w, (size_t)m * 48), o_oct = pk.add(last->octave, (size_t)m * 4);
-    const size_t o_qd = pk.add(last->desc, (size_t)m * 32), o_val = pk.add(last->valid, (size_t)m);
-    const size_t o_sf = pk.add(scale_factors_lsd, (size_t)num_levels_lsd * 4);
-    size_t oq[6];
-    for (int k = 0; k < 6; ++k) oq[k] = pk.reserve((size_t)m * 4);
-    const size_t o_r = pk.reserve((size_t)m * 4), o_mn = pk.reserve((size_t)m * 4), o_mx = pk.reserve((size_t)m * 4);
-    const size_t o_qv = pk.reserve((size_t)m);
-    const size_t o_choice = pk.reserve((size_t)m * 4), o_matched = pk.reserve((size_t)n * 4), o_num = pk.reserve(4);
-    const size_t o_job = pk.reserve(sizeof(LineMatchJob)), o_pjob = pk.reserve(sizeof(ProjectJob));
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    bind_frame_lines(d, fo, curr, J);
+    plp_frame_lines f = *curr;
+    f.ratio_level = nullptr;  // no ratio test here: the matcher never reads the ratio levels
+    add_frame_lines(lay, f, J);
     P.n_last = m;
-    P.pos_w = Packer::at<double>(d, o_pw);
-    P.octave = Packer::at<int32_t>(d, o_oct);
-    P.valid = Packer::at<uint8_t>(d, o_val);
+    lay.in(P.pos_w, last->pos_w, (size_t)m * 6);
+    lay.in(P.octave, last->octave, m);
+    lay.in(J.qdesc, last->desc, (size_t)m * 32);
+    lay.in(P.valid, last->valid, m);
+    const float *d_sf;
+    lay.in(d_sf, scale_factors_lsd, num_levels_lsd);
     for (int r = 0; r < 3; ++r)
         for (int c = 0; c < 4; ++c) P.pose_cw[r * 4 + c] = pose_cw_curr[r * 4 + c];
     motion_assumption(*cam, pose_cw_curr, pose_cw_last, &P.assume_forward, &P.assume_backward);
-    P.qx = Packer::at<float>(d, oq[0]);
-    P.qy = Packer::at<float>(d, oq[1]);
-    P.qxr = Packer::at<float>(d, oq[2]);
-    P.qx2 = Packer::at<float>(d, oq[3]);
-    P.qy2 = Packer::at<float>(d, oq[4]);
-    P.qxr2 = Packer::at<float>(d, oq[5]);
-    P.qradius = Packer::at<float>(d, o_r);
-    P.qmin = Packer::at<int32_t>(d, o_mn);
-    P.qmax = Packer::at<int32_t>(d, o_mx);
-    P.qvalid = Packer::at<uint8_t>(d, o_qv);
     J.m = m;
-    J.q_spx = P.qx;
-    J.q_spy = P.qy;
-    J.q_xr_sp = P.qxr;
-    J.q_epx = P.qx2;
-    J.q_epy = P.qy2;
-    J.q_xr_ep = P.qxr2;
-    J.qradius = P.qradius;
-    J.qmin = P.qmin;
-    J.qmax = P.qmax;
-    J.qdesc = Packer::at<uint8_t>(d, o_qd);
-    J.qvalid = P.qvalid;
-    J.choice = Packer::at<int32_t>(d, o_choice);
-    J.matched_out = Packer::at<int32_t>(d, o_matched);
-    J.num_matches = Packer::at<uint32_t>(d, o_num);
-    J.ratio_level = nullptr;
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_job, &J, sizeof(J), cudaMemcpyHostToDevice, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_pjob, &P, sizeof(P), cudaMemcpyHostToDevice, ctx->stream));
-    PLP_TRY(launch_project_lines(ctx, Packer::at<ProjectJob>(d, o_pjob), 1, m, *cam, Packer::at<float>(d, o_sf),
-                                 num_levels_lsd, margin));
-    PLP_TRY(launch_line_match(ctx, Packer::at<LineMatchJob>(d, o_job), 1, 0, 0.0f, cam->setup_type == 2));
+    const LineMatchJob *d_job;
+    const ProjectJob *d_pjob;
+    lay.in(d_job, &J, 1);
+    lay.in(d_pjob, &P, 1);
+    // the projection pre-pass writes the queries the matcher reads
+    lay.out(P.qx, m);
+    lay.out(P.qy, m);
+    lay.out(P.qxr, m);
+    lay.out(P.qx2, m);
+    lay.out(P.qy2, m);
+    lay.out(P.qxr2, m);
+    lay.out(P.qradius, m);
+    lay.out(P.qmin, m);
+    lay.out(P.qmax, m);
+    lay.out(P.qvalid, m);
+    lay.alias(J.q_spx, P.qx);
+    lay.alias(J.q_spy, P.qy);
+    lay.alias(J.q_xr_sp, P.qxr);
+    lay.alias(J.q_epx, P.qx2);
+    lay.alias(J.q_epy, P.qy2);
+    lay.alias(J.q_xr_ep, P.qxr2);
+    lay.alias(J.qradius, P.qradius);
+    lay.alias(J.qmin, P.qmin);
+    lay.alias(J.qmax, P.qmax);
+    lay.alias(J.qvalid, P.qvalid);
+    lay.out(J.choice, m);
+    lay.out(J.matched_out, n);
+    lay.out(J.num_matches, 1);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_TRY(launch_project_lines(ctx, d_pjob, 1, m, *cam, d_sf, num_levels_lsd, margin));
+    PLP_TRY(launch_line_match(ctx, d_job, 1, 0, 0.0f, cam->setup_type == 2));
     uint32_t num = 0;
-    PLP_CUDA_TRY(cudaMemcpyAsync(matched_last_idx_out, d + o_matched, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(&num, d + o_num, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(matched_last_idx_out, J.matched_out, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(&num, J.num_matches, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (num_matches_out) *num_matches_out = num;
     return PLP_OK;
@@ -1105,41 +1056,32 @@ plp_status plp_match_frame_and_keyframe(plp_ctx *ctx, const plp_frame_points *fr
         qmin[i] = lvl - 1;
         qmax[i] = lvl + 1;
     }
-    Packer pk;
+    Layout lay;
     PointMatchJob J;
     memset(&J, 0, sizeof(J));
-    size_t fo[7];
-    pack_frame_points(pk, frm, J, fo);
-    const size_t o_qx = pk.add(q->reproj_x, (size_t)m * 4), o_qy = pk.add(q->reproj_y, (size_t)m * 4);
-    const size_t o_r = pk.add(radius.data(), (size_t)m * 4);
-    const size_t o_mn = pk.add(qmin.data(), (size_t)m * 4), o_mx = pk.add(qmax.data(), (size_t)m * 4);
-    const size_t o_qa = pk.add(q_angle, (size_t)m * 4);
-    const size_t o_qd = pk.add(q->desc, (size_t)m * 32), o_qv = pk.add(q->valid, (size_t)m);
-    const size_t o_choice = pk.reserve((size_t)m * 4), o_matched = pk.reserve((size_t)n * 4), o_num = pk.reserve(4);
-    const size_t o_job = pk.reserve(sizeof(PointMatchJob));
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    bind_frame_points(d, fo, J);
-    J.x_right = nullptr;  // no stereo gate in match_frame_and_keyframe
+    plp_frame_points f = *frm;
+    f.x_right = nullptr;  // no stereo gate in match_frame_and_keyframe
+    add_frame_points(lay, f, J);
     J.m = m;
-    J.qx = Packer::at<float>(d, o_qx);
-    J.qy = Packer::at<float>(d, o_qy);
-    J.qxr = nullptr;
-    J.qradius = Packer::at<float>(d, o_r);
-    J.qmin = Packer::at<int32_t>(d, o_mn);
-    J.qmax = Packer::at<int32_t>(d, o_mx);
-    J.qangle = q_angle ? Packer::at<float>(d, o_qa) : nullptr;
-    J.qdesc = Packer::at<uint8_t>(d, o_qd);
-    J.qvalid = q->valid ? Packer::at<uint8_t>(d, o_qv) : nullptr;
-    J.choice = Packer::at<int32_t>(d, o_choice);
-    J.matched_out = Packer::at<int32_t>(d, o_matched);
-    J.num_matches = Packer::at<uint32_t>(d, o_num);
+    lay.in(J.qx, q->reproj_x, m);
+    lay.in(J.qy, q->reproj_y, m);
+    lay.in(J.qradius, radius.data(), m);
+    lay.in(J.qmin, qmin.data(), m);
+    lay.in(J.qmax, qmax.data(), m);
+    lay.in(J.qangle, q_angle, m);
+    lay.in(J.qdesc, q->desc, (size_t)m * 32);
+    lay.in(J.qvalid, q->valid, m);
     J.hamm_thr_p1 = hamm_dist_thr + 1u;
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_job, &J, sizeof(J), cudaMemcpyHostToDevice, ctx->stream));
-    PLP_TRY(launch_point_match(ctx, Packer::at<PointMatchJob>(d, o_job), 1, n, *grid, 0, 0.0f, check_orientation));
+    const PointMatchJob *d_job;
+    lay.in(d_job, &J, 1);
+    lay.out(J.choice, m);
+    lay.out(J.matched_out, n);
+    lay.out(J.num_matches, 1);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_TRY(launch_point_match(ctx, d_job, 1, n, *grid, 0, 0.0f, check_orientation));
     uint32_t num = 0;
-    PLP_CUDA_TRY(cudaMemcpyAsync(matched_kf_idx_out, d + o_matched, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(&num, d + o_num, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(matched_kf_idx_out, J.matched_out, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(&num, J.num_matches, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (num_matches_out) *num_matches_out = num;
     return PLP_OK;
@@ -1168,41 +1110,33 @@ plp_status plp_match_frame_and_keyframe_line(plp_ctx *ctx, const plp_frame_lines
         qmin[i] = lvl - 1;
         qmax[i] = lvl + 1;
     }
-    Packer pk;
+    Layout lay;
     LineMatchJob J;
     memset(&J, 0, sizeof(J));
-    size_t fo[11];
-    pack_frame_lines(pk, frm, fo);
-    const size_t o1 = pk.add(q->sp_x, (size_t)m * 4), o2 = pk.add(q->sp_y, (size_t)m * 4);
-    const size_t o3 = pk.add(q->ep_x, (size_t)m * 4), o4 = pk.add(q->ep_y, (size_t)m * 4);
-    const size_t o_r = pk.add(radius.data(), (size_t)m * 4);
-    const size_t o_mn = pk.add(qmin.data(), (size_t)m * 4), o_mx = pk.add(qmax.data(), (size_t)m * 4);
-    const size_t o_qd = pk.add(q->desc, (size_t)m * 32), o_qv = pk.add(q->valid, (size_t)m);
-    const size_t o_choice = pk.reserve((size_t)m * 4), o_matched = pk.reserve((size_t)n * 4), o_num = pk.reserve(4);
-    const size_t o_job = pk.reserve(sizeof(LineMatchJob));
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    bind_frame_lines(d, fo, frm, J);
+    plp_frame_lines f = *frm;
+    f.ratio_level = nullptr;  // no ratio test here: the matcher never reads the ratio levels
+    add_frame_lines(lay, f, J);
     J.m = m;
-    J.q_spx = Packer::at<float>(d, o1);
-    J.q_spy = Packer::at<float>(d, o2);
-    J.q_epx = Packer::at<float>(d, o3);
-    J.q_epy = Packer::at<float>(d, o4);
-    J.qradius = Packer::at<float>(d, o_r);
-    J.qmin = Packer::at<int32_t>(d, o_mn);
-    J.qmax = Packer::at<int32_t>(d, o_mx);
-    J.qdesc = Packer::at<uint8_t>(d, o_qd);
-    J.qvalid = q->valid ? Packer::at<uint8_t>(d, o_qv) : nullptr;
-    J.choice = Packer::at<int32_t>(d, o_choice);
-    J.matched_out = Packer::at<int32_t>(d, o_matched);
-    J.num_matches = Packer::at<uint32_t>(d, o_num);
-    J.ratio_level = nullptr;
+    lay.in(J.q_spx, q->sp_x, m);
+    lay.in(J.q_spy, q->sp_y, m);
+    lay.in(J.q_epx, q->ep_x, m);
+    lay.in(J.q_epy, q->ep_y, m);
+    lay.in(J.qradius, radius.data(), m);
+    lay.in(J.qmin, qmin.data(), m);
+    lay.in(J.qmax, qmax.data(), m);
+    lay.in(J.qdesc, q->desc, (size_t)m * 32);
+    lay.in(J.qvalid, q->valid, m);
     J.hamm_thr_p1 = hamm_dist_thr + 1u;
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_job, &J, sizeof(J), cudaMemcpyHostToDevice, ctx->stream));
-    PLP_TRY(launch_line_match(ctx, Packer::at<LineMatchJob>(d, o_job), 1, 0, 0.0f, 0));
+    const LineMatchJob *d_job;
+    lay.in(d_job, &J, 1);
+    lay.out(J.choice, m);
+    lay.out(J.matched_out, n);
+    lay.out(J.num_matches, 1);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_TRY(launch_line_match(ctx, d_job, 1, 0, 0.0f, 0));
     uint32_t num = 0;
-    PLP_CUDA_TRY(cudaMemcpyAsync(matched_kf_idx_out, d + o_matched, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(&num, d + o_num, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(matched_kf_idx_out, J.matched_out, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(&num, J.num_matches, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (num_matches_out) *num_matches_out = num;
     return PLP_OK;
@@ -1220,32 +1154,27 @@ plp_status plp_match_brute_force(plp_ctx *ctx, const uint8_t *frm_desc, const fl
     PLP_REQUIRE(frm_desc && kf_desc, "descriptors");
     PLP_REQUIRE(!check_orientation || (frm_angle && kf_angle), "angles required for the orientation check");
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
+    Layout lay;
     BruteJob J;
     memset(&J, 0, sizeof(J));
-    const size_t o1 = pk.add(frm_desc, (size_t)n_frm * 32), o2 = pk.add(frm_angle, (size_t)n_frm * 4);
-    const size_t o3 = pk.add(kf_desc, (size_t)n_kf * 32), o4 = pk.add(kf_angle, (size_t)n_kf * 4);
-    const size_t o5 = pk.add(kf_valid, (size_t)n_kf);
-    const size_t o_choice = pk.reserve((size_t)n_kf * 4), o_matched = pk.reserve((size_t)n_frm * 4), o_num = pk.reserve(4);
-    const size_t o_job = pk.reserve(sizeof(BruteJob));
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
     J.n_frm = n_frm;
-    J.frm_desc = Packer::at<uint8_t>(d, o1);
-    J.frm_angle = Packer::at<float>(d, o2);
+    lay.in(J.frm_desc, frm_desc, (size_t)n_frm * 32);
+    lay.in(J.frm_angle, frm_angle, n_frm);
     J.n_kf = n_kf;
-    J.kf_desc = Packer::at<uint8_t>(d, o3);
-    J.kf_angle = Packer::at<float>(d, o4);
-    J.kf_valid = Packer::at<uint8_t>(d, o5);
-    J.choice = Packer::at<int32_t>(d, o_choice);
-    J.matched_out = Packer::at<int32_t>(d, o_matched);
-    J.num_matches = Packer::at<uint32_t>(d, o_num);
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_job, &J, sizeof(J), cudaMemcpyHostToDevice, ctx->stream));
-    PLP_TRY(launch_brute_match(ctx, Packer::at<BruteJob>(d, o_job), 1, n_frm, lowe_ratio, check_orientation));
+    lay.in(J.kf_desc, kf_desc, (size_t)n_kf * 32);
+    lay.in(J.kf_angle, kf_angle, n_kf);
+    lay.in(J.kf_valid, kf_valid, n_kf);
+    const BruteJob *d_job;
+    lay.in(d_job, &J, 1);
+    lay.out(J.choice, n_kf);
+    lay.out(J.matched_out, n_frm);
+    lay.out(J.num_matches, 1);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_TRY(launch_brute_match(ctx, d_job, 1, n_frm, lowe_ratio, check_orientation));
     uint32_t num = 0;
-    PLP_CUDA_TRY(cudaMemcpyAsync(matched_kf_idx_in_frm_out, d + o_matched, (size_t)n_frm * 4, cudaMemcpyDeviceToHost,
+    PLP_CUDA_TRY(cudaMemcpyAsync(matched_kf_idx_in_frm_out, J.matched_out, (size_t)n_frm * 4, cudaMemcpyDeviceToHost,
                                  ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(&num, d + o_num, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(&num, J.num_matches, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (num_matches_out) *num_matches_out = num;
     return PLP_OK;
@@ -1305,53 +1234,42 @@ plp_status plp_match_for_triangulation(plp_ctx *ctx, const plp_keyframe_points *
         for (size_t i = 0; i < n1; ++i) st1[i] = 0 <= kf1->x_right[i];
     if (kf2->x_right)
         for (size_t i = 0; i < n2; ++i) st2[i] = 0 <= kf2->x_right[i];
-    Packer pk;
+    Layout lay;
     TriJob J;
     memset(&J, 0, sizeof(J));
-    const size_t o_d1 = pk.add(kf1->desc, n1 * 32), o_d2 = pk.add(kf2->desc, n2 * 32);
-    const size_t o_a1 = pk.add(kf1->angle, n1 * 4), o_a2 = pk.add(kf2->angle, n2 * 4);
-    const size_t o_o1 = pk.add(kf1->octave, n1 * 4);
-    const size_t o_b1 = pk.add(kf1->bearings, n1 * 24), o_b2 = pk.add(kf2->bearings, n2 * 24);
-    const size_t o_l2 = pk.add(kf2->has_landmark, n2);
-    const size_t o_s1 = pk.add(st1.data(), n1), o_s2 = pk.add(st2.data(), n2);
-    const size_t o_q1 = pk.add(seq_idx1.data(), (size_t)P * 4), o_qb = pk.add(seq_cbeg.data(), (size_t)P * 4);
-    const size_t o_qe = pk.add(seq_cend.data(), (size_t)P * 4), o_c2 = pk.add(cand2.data(), cand2.size() * 4);
-    const size_t o_sf = pk.add(scale_factors_1, (size_t)num_levels * 4);
-    const size_t o_choice = pk.reserve((size_t)P * 4), o_matched = pk.reserve(n1 * 4), o_num = pk.reserve(4);
-    const size_t o_job = pk.reserve(sizeof(TriJob));
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
     J.n1 = (int)n1;
     J.n2 = (int)n2;
     J.num_seq = P;
-    J.desc1 = Packer::at<uint8_t>(d, o_d1);
-    J.desc2 = Packer::at<uint8_t>(d, o_d2);
-    J.angle1 = kf1->angle ? Packer::at<float>(d, o_a1) : nullptr;
-    J.angle2 = kf2->angle ? Packer::at<float>(d, o_a2) : nullptr;
-    J.octave1 = Packer::at<int32_t>(d, o_o1);
-    J.bearing1 = Packer::at<double>(d, o_b1);
-    J.bearing2 = Packer::at<double>(d, o_b2);
-    J.has_lm2 = Packer::at<uint8_t>(d, o_l2);
-    J.stereo1 = Packer::at<uint8_t>(d, o_s1);
-    J.stereo2 = Packer::at<uint8_t>(d, o_s2);
-    J.seq_idx1 = Packer::at<int32_t>(d, o_q1);
-    J.seq_cbeg = Packer::at<int32_t>(d, o_qb);
-    J.seq_cend = Packer::at<int32_t>(d, o_qe);
-    J.cand2 = Packer::at<int32_t>(d, o_c2);
-    J.scale_factors1 = Packer::at<float>(d, o_sf);
+    lay.in(J.desc1, kf1->desc, n1 * 32);
+    lay.in(J.desc2, kf2->desc, n2 * 32);
+    lay.in(J.angle1, kf1->angle, n1);
+    lay.in(J.angle2, kf2->angle, n2);
+    lay.in(J.octave1, kf1->octave, n1);
+    lay.in(J.bearing1, kf1->bearings, n1 * 3);
+    lay.in(J.bearing2, kf2->bearings, n2 * 3);
+    lay.in(J.has_lm2, kf2->has_landmark, n2);
+    lay.in(J.stereo1, st1.data(), n1);
+    lay.in(J.stereo2, st2.data(), n2);
+    lay.in(J.seq_idx1, seq_idx1.data(), P);
+    lay.in(J.seq_cbeg, seq_cbeg.data(), P);
+    lay.in(J.seq_cend, seq_cend.data(), P);
+    lay.in(J.cand2, cand2.data(), cand2.size());
+    lay.in(J.scale_factors1, scale_factors_1, num_levels);
     for (int k = 0; k < 9; ++k) J.E[k] = E_12[k];
     for (int k = 0; k < 3; ++k) J.epipole[k] = epipole_bearing_in_2[k];
-    J.choice = Packer::at<int32_t>(d, o_choice);
-    J.matched_out = Packer::at<int32_t>(d, o_matched);
-    J.num_matches = Packer::at<uint32_t>(d, o_num);
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_job, &J, sizeof(J), cudaMemcpyHostToDevice, ctx->stream));
+    const TriJob *d_job;
+    lay.in(d_job, &J, 1);
+    lay.out(J.choice, P);
+    lay.out(J.matched_out, n1);
+    lay.out(J.num_matches, 1);
+    PLP_TRY(lay.upload(ctx, 0));
     const size_t smem = (size_t)n2 * 8 + (kHistLen + 4) * 4 + kHistLen + 16;
     PLP_SMEM_OPTIN(triangulation_match_kernel, smem);
-    PLP_LAUNCH(ctx, triangulation_match_kernel, 1, kThreads, smem, Packer::at<TriJob>(d, o_job), (int)n2, check_orientation);
+    PLP_LAUNCH(ctx, triangulation_match_kernel, 1, kThreads, smem, d_job, (int)n2, check_orientation);
     PLP_CHECK_LAUNCH();
     uint32_t num = 0;
-    PLP_CUDA_TRY(cudaMemcpyAsync(matched_idx2_in_1_out, d + o_matched, n1 * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(&num, d + o_num, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(matched_idx2_in_1_out, J.matched_out, n1 * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(&num, J.num_matches, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (num_matches_out) *num_matches_out = num;
     return PLP_OK;
@@ -1366,15 +1284,18 @@ plp_status plp_landmark_compute_descriptor_batch(plp_ctx *ctx, const uint8_t *de
     PLP_REQUIRE(offsets[0] == 0 && total >= 0 && (total == 0 || descs), "offsets");
     for (int i = 0; i < num_landmarks; ++i) PLP_REQUIRE(offsets[i] <= offsets[i + 1], "offsets must ascend");
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
-    const size_t o_d = pk.add(descs, (size_t)total * 32), o_o = pk.add(offsets, (size_t)(num_landmarks + 1) * 4);
-    const size_t o_b = pk.reserve((size_t)num_landmarks * 4);
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    PLP_LAUNCH(ctx, median_descriptor_kernel, div_up(num_landmarks, kMedWarps), kMedWarps * 32, 0, Packer::at<uint8_t>(d, o_d),
-               Packer::at<int32_t>(d, o_o), num_landmarks, Packer::at<int32_t>(d, o_b));
+    Layout lay;
+    const uint8_t *dd;
+    const int32_t *doff;
+    int32_t *dbest;
+    lay.in(dd, descs, (size_t)total * 32);
+    lay.in(doff, offsets, (size_t)num_landmarks + 1);
+    lay.out(dbest, num_landmarks);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_LAUNCH(ctx, median_descriptor_kernel, div_up(num_landmarks, kMedWarps), kMedWarps * 32, 0, dd, doff,
+               num_landmarks, dbest);
     PLP_CHECK_LAUNCH();
-    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, d + o_b, (size_t)num_landmarks * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(best_idx_out, dbest, (size_t)num_landmarks * 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return PLP_OK;
 }

@@ -12,6 +12,7 @@
 // the adapter instead).
 #include "common.cuh"
 #include "match_kernels.cuh"
+#include "pack.cuh"
 #include "pose_kernels.cuh"
 
 namespace plp {
@@ -257,51 +258,39 @@ plp_status plp_tracker_create(plp_ctx *ctx, const plp_camera *cam, const plp_gri
         t->inv_level_sigma_sq[l] = inv_level_sigma_sq[l];
     }
     const size_t B = max_batch, C = kp_capacity, M = max_last_points;
-    size_t off = 0;
-    auto take = [&](size_t bytes) {
-        const size_t o = off;
-        off += (bytes + 255) & ~(size_t)255;
-        return o;
-    };
-    const size_t o_sf = take(16 * 4);
-    const size_t o_x = take(B * C * 4), o_y = take(B * C * 4), o_ang = take(B * C * 4), o_oct = take(B * C * 4);
-    const size_t o_qx = take(B * M * 4), o_qy = take(B * M * 4), o_qxr = take(B * M * 4), o_qr = take(B * M * 4);
-    const size_t o_qmin = take(B * M * 4), o_qmax = take(B * M * 4), o_qv = take(B * M), o_choice = take(B * M * 4);
-    const size_t o_nm = take(B * 4), o_pj = take(2 * B * sizeof(ProjectJob)), o_mj = take(2 * B * sizeof(PointMatchJob));
-    const size_t o_poj = take(B * sizeof(PoseJob)), o_obs = take(B * C * sizeof(plp_pt_obs)), o_okp = take(B * C * 4);
-    const size_t o_oout = take(B * C);
-    if (cudaMalloc((void **)&t->d_block, off) != cudaSuccess) {
-        set_error("tracker: cudaMalloc(%zu) failed", off);
+    TrackDev &T = t->dev;
+    memset(&T, 0, sizeof(T));
+    Layout lay;
+    lay.out(t->d_scale_factors, 16);
+    lay.out(T.x, B * C);
+    lay.out(T.y, B * C);
+    lay.out(T.angle, B * C);
+    lay.out(T.octave, B * C);
+    lay.out(T.qx, B * M);
+    lay.out(T.qy, B * M);
+    lay.out(T.qxr, B * M);
+    lay.out(T.qradius, B * M);
+    lay.out(T.qmin, B * M);
+    lay.out(T.qmax, B * M);
+    lay.out(T.qvalid, B * M);
+    lay.out(T.choice, B * M);
+    lay.out(T.num_matches, B);
+    lay.out(T.pjobs, 2 * B);
+    lay.out(T.mjobs, 2 * B);
+    lay.out(T.posejobs, B);
+    lay.out(T.obs, B * C);
+    lay.out(T.obs_kp, B * C);
+    lay.out(T.obs_outlier, B * C);
+    if (cudaMalloc((void **)&t->d_block, lay.bytes()) != cudaSuccess) {
+        set_error("tracker: cudaMalloc(%zu) failed", lay.bytes());
         delete t;
         return PLP_ERR_CUDA;
     }
-    uint8_t *d = t->d_block;
-    t->d_scale_factors = (float *)(d + o_sf);
+    lay.bind(t->d_block);
     cudaMemcpy(t->d_scale_factors, t->scale_factors, num_levels * 4, cudaMemcpyHostToDevice);
-    TrackDev &T = t->dev;
-    memset(&T, 0, sizeof(T));
     T.cap = kp_capacity;
     T.num_levels = num_levels;
     T.max_last = max_last_points;
-    T.x = (float *)(d + o_x);
-    T.y = (float *)(d + o_y);
-    T.angle = (float *)(d + o_ang);
-    T.octave = (int32_t *)(d + o_oct);
-    T.qx = (float *)(d + o_qx);
-    T.qy = (float *)(d + o_qy);
-    T.qxr = (float *)(d + o_qxr);
-    T.qradius = (float *)(d + o_qr);
-    T.qmin = (int32_t *)(d + o_qmin);
-    T.qmax = (int32_t *)(d + o_qmax);
-    T.qvalid = d + o_qv;
-    T.choice = (int32_t *)(d + o_choice);
-    T.num_matches = (uint32_t *)(d + o_nm);
-    T.pjobs = (ProjectJob *)(d + o_pj);
-    T.mjobs = (PointMatchJob *)(d + o_mj);
-    T.posejobs = (PoseJob *)(d + o_poj);
-    T.obs = (plp_pt_obs *)(d + o_obs);
-    T.obs_kp = (int32_t *)(d + o_okp);
-    T.obs_outlier = d + o_oout;
     for (int l = 0; l < 16; ++l) T.inv_level_sigma_sq[l] = l < num_levels ? inv_level_sigma_sq[l] : 1.0f;
     *out = t;
     return PLP_OK;

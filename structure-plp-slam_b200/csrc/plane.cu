@@ -36,44 +36,37 @@ plp_status plp_plane_ransac(plp_ctx *ctx, const double *pos_w, const uint8_t *va
     for (long long i = 0; i < (long long)num_iter * sample_size; ++i)
         PLP_REQUIRE(samples[i] >= 0 && samples[i] < n, "sample index out of range");
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
+    Layout lay;
     const size_t N = (size_t)n, K = (size_t)num_iter;
-    const size_t o_pos = pk.add(pos_w, N * 24), o_val = pk.add(valid, N);
-    const size_t o_smp = pk.add(samples, K * (size_t)sample_size * 4);
-    const size_t o_eq = pk.add(eq_inout, 32), o_pe = pk.add(plane_error_inout, 8);
-    const size_t o_eqs = pk.reserve(K * 32), o_eqr = pk.reserve(K * 32), o_res = pk.reserve(K * 8), o_err = pk.reserve(K * 8);
-    const size_t o_el = pk.reserve(K * 4), o_cnt = pk.reserve(K * 4), o_flag = pk.reserve(K * N), o_idx = pk.reserve(K * N * 4);
-    const size_t o_inl = pk.reserve(N), o_st = pk.reserve(4);
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
     PlaneJob J;
-    J.pos = Packer::at<double>(d, o_pos);
-    J.valid = Packer::at<uint8_t>(d, o_val);
-    J.samples = Packer::at<int32_t>(d, o_smp);
+    lay.in(J.pos, pos_w, N * 3);
+    lay.in(J.valid, valid, N);
+    lay.in(J.samples, samples, K * (size_t)sample_size);
+    lay.in(J.eq, eq_inout, 4);
+    lay.in(J.plane_err, plane_error_inout, 1);
+    lay.out(J.eq_s, K * 4);
+    lay.out(J.eq_r, K * 4);
+    lay.out(J.res, K);
+    lay.out(J.err, K);
+    lay.out(J.elig, K);
+    lay.out(J.cnt, K);
+    lay.out(J.flag, K * N);
+    lay.out(J.idx, K * N);
+    lay.out(J.inlier, N);
+    lay.out(J.status, 1);
     J.n = n;
     J.num_iter = num_iter;
     J.sample_size = sample_size;
     J.cfg = *cfg;
-    J.eq_s = Packer::at<double>(d, o_eqs);
-    J.eq_r = Packer::at<double>(d, o_eqr);
-    J.res = Packer::at<double>(d, o_res);
-    J.err = Packer::at<double>(d, o_err);
-    J.elig = Packer::at<int32_t>(d, o_el);
-    J.cnt = Packer::at<int32_t>(d, o_cnt);
-    J.flag = Packer::at<uint8_t>(d, o_flag);
-    J.idx = Packer::at<int32_t>(d, o_idx);
-    J.eq = Packer::at<double>(d, o_eq);
-    J.plane_err = Packer::at<double>(d, o_pe);
-    J.inlier = Packer::at<uint8_t>(d, o_inl);
-    J.status = Packer::at<int32_t>(d, o_st);
+    PLP_TRY(lay.upload(ctx, 0));
     PLP_LAUNCH(ctx, plane_hypothesis_kernel, num_iter, kPlThreads, 0, J);
     PLP_CHECK_LAUNCH();
     PLP_LAUNCH(ctx, plane_select_kernel, 1, kPlThreads, 0, J);
     PLP_CHECK_LAUNCH();
-    PLP_CUDA_TRY(cudaMemcpyAsync(eq_inout, d + o_eq, 32, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(plane_error_inout, d + o_pe, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(inlier_out, d + o_inl, N, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(status_out, d + o_st, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(eq_inout, J.eq, 32, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(plane_error_inout, J.plane_err, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(inlier_out, J.inlier, N, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(status_out, J.status, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return PLP_OK;
 }

@@ -102,27 +102,31 @@ plp_status plp_pose_optimize_batch(plp_ctx *ctx, const plp_camera *cam, int batc
         max_edges = e > max_edges ? e : max_edges;
     }
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    Packer pk;
-    std::vector<int32_t> zero_off(batch + 1, 0);
-    const size_t o_T = pk.add(T_in, (size_t)batch * 128);
-    const size_t o_pts = pk.add(n_pts ? (const void *)pts : (const void *)zero_off.data(), n_pts ? (size_t)n_pts * sizeof(plp_pt_obs) : 8);
-    const size_t o_po = pk.add(pt_off, (size_t)(batch + 1) * 4);
-    const size_t o_lines = n_lines ? pk.add(lines, (size_t)n_lines * sizeof(plp_line_obs)) : Packer::kNone;
-    const size_t o_lo = n_lines ? pk.add(line_off, (size_t)(batch + 1) * 4) : Packer::kNone;
-    const size_t o_To = pk.reserve((size_t)batch * 128);
-    const size_t o_pout = pk.reserve((size_t)n_pts + 8), o_lout = pk.reserve((size_t)n_lines + 8);
-    const size_t o_inl = pk.reserve((size_t)batch * 4);
-    uint8_t *d;
-    PLP_TRY(pk.upload(ctx, 0, &d));
-    PLP_TRY(plp_pose_optimize_batch_dev(ctx, cam, batch, Packer::at<double>(d, o_T), Packer::at<plp_pt_obs>(d, o_pts),
-                                        Packer::at<int32_t>(d, o_po), Packer::at<plp_line_obs>(d, o_lines),
-                                        Packer::at<int32_t>(d, o_lo), max_edges, cfg, Packer::at<double>(d, o_To),
-                                        Packer::at<uint8_t>(d, o_pout), n_lines ? Packer::at<uint8_t>(d, o_lout) : nullptr,
-                                        Packer::at<int32_t>(d, o_inl), nullptr));
-    PLP_CUDA_TRY(cudaMemcpyAsync(T_out, d + o_To, (size_t)batch * 128, cudaMemcpyDeviceToHost, ctx->stream));
-    if (n_pts) PLP_CUDA_TRY(cudaMemcpyAsync(pt_outlier, d + o_pout, (size_t)n_pts, cudaMemcpyDeviceToHost, ctx->stream));
-    if (n_lines) PLP_CUDA_TRY(cudaMemcpyAsync(line_outlier, d + o_lout, (size_t)n_lines, cudaMemcpyDeviceToHost, ctx->stream));
-    PLP_CUDA_TRY(cudaMemcpyAsync(n_inliers, d + o_inl, (size_t)batch * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    Layout lay;
+    static const plp_pt_obs no_pts{};  // the batch entry point takes a non-null point array even without points
+    const double *d_T;
+    const plp_pt_obs *d_pts;
+    const int32_t *d_po, *d_lo;
+    const plp_line_obs *d_lines;
+    double *d_To;
+    uint8_t *d_pout, *d_lout = nullptr;
+    int32_t *d_inl;
+    lay.in(d_T, T_in, (size_t)batch * 16);
+    lay.in(d_pts, n_pts ? pts : &no_pts, n_pts ? (size_t)n_pts : 1);
+    lay.in(d_po, pt_off, (size_t)batch + 1);
+    lay.in(d_lines, lines, n_lines);
+    lay.in(d_lo, n_lines ? line_off : nullptr, (size_t)batch + 1);
+    lay.out(d_To, (size_t)batch * 16);
+    lay.out(d_pout, (size_t)n_pts + 8);
+    if (n_lines) lay.out(d_lout, (size_t)n_lines + 8);
+    lay.out(d_inl, batch);
+    PLP_TRY(lay.upload(ctx, 0));
+    PLP_TRY(plp_pose_optimize_batch_dev(ctx, cam, batch, d_T, d_pts, d_po, d_lines, d_lo, max_edges, cfg, d_To, d_pout,
+                                        d_lout, d_inl, nullptr));
+    PLP_CUDA_TRY(cudaMemcpyAsync(T_out, d_To, (size_t)batch * 128, cudaMemcpyDeviceToHost, ctx->stream));
+    if (n_pts) PLP_CUDA_TRY(cudaMemcpyAsync(pt_outlier, d_pout, (size_t)n_pts, cudaMemcpyDeviceToHost, ctx->stream));
+    if (n_lines) PLP_CUDA_TRY(cudaMemcpyAsync(line_outlier, d_lout, (size_t)n_lines, cudaMemcpyDeviceToHost, ctx->stream));
+    PLP_CUDA_TRY(cudaMemcpyAsync(n_inliers, d_inl, (size_t)batch * 4, cudaMemcpyDeviceToHost, ctx->stream));
     PLP_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return PLP_OK;
 }

@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "pack.cuh"
 
 using namespace plp;
 
@@ -273,25 +274,28 @@ plp_status plp_stereo_compute(plp_ctx *ctx, const plp_orb *left, const plp_orb *
     const int cap = plp_orb_capacity(left);
     PLP_REQUIRE(n_l <= cap && n_r <= cap, "more keypoints than the extractor's capacity");
     PLP_CUDA_TRY(cudaSetDevice(ctx->device));
-    const size_t kb = (size_t)cap * sizeof(plp_keypoint), db = (size_t)cap * 32;
-    const size_t o_kl = 0, o_kr = o_kl + kb, o_dl = o_kr + kb, o_dr = o_dl + db, o_n = o_dr + db, o_x = o_n + 16,
-                 o_d = o_x + (size_t)cap * 4, o_b = o_d + (size_t)cap * 4, total = o_b + (size_t)cap * 4;
-    uint8_t *d = nullptr;
-    PLP_TRY(ctx_scratch(ctx, 3, total, (void **)&d));
+    Layout lay;
     const int32_t n2[2] = {n_l, n_r};
+    const plp_keypoint *dkl, *dkr;
+    const uint8_t *ddl, *ddr;
+    const int32_t *dn;
+    float *dx, *dd;
+    int32_t *db;
+    lay.in(dkl, kp_l, n_l);
+    lay.in(dkr, kp_r, n_r);
+    lay.in(ddl, desc_l, (size_t)n_l * 32);
+    lay.in(ddr, desc_r, (size_t)n_r * 32);
+    lay.in(dn, n2, 2);
+    lay.out(dx, n_l);
+    lay.out(dd, n_l);
+    lay.out(db, n_l);
+    PLP_TRY(lay.upload(ctx, 3));
+    PLP_TRY(plp_stereo_compute_batch_dev(ctx, left, right, 1, dkl, ddl, dn, dkr, ddr, dn + 1, focal_x_baseline,
+                                         true_baseline, dx, dd, db));
     cudaStream_t s = ctx->stream;
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_kl, kp_l, (size_t)n_l * sizeof(plp_keypoint), cudaMemcpyHostToDevice, s));
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_kr, kp_r, (size_t)n_r * sizeof(plp_keypoint), cudaMemcpyHostToDevice, s));
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_dl, desc_l, (size_t)n_l * 32, cudaMemcpyHostToDevice, s));
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_dr, desc_r, (size_t)n_r * 32, cudaMemcpyHostToDevice, s));
-    PLP_CUDA_TRY(cudaMemcpyAsync(d + o_n, n2, 8, cudaMemcpyHostToDevice, s));
-    PLP_TRY(plp_stereo_compute_batch_dev(ctx, left, right, 1, (const plp_keypoint *)(d + o_kl), d + o_dl,
-                                         (const int32_t *)(d + o_n), (const plp_keypoint *)(d + o_kr), d + o_dr,
-                                         (const int32_t *)(d + o_n + 4), focal_x_baseline, true_baseline, (float *)(d + o_x),
-                                         (float *)(d + o_d), (int32_t *)(d + o_b)));
-    PLP_CUDA_TRY(cudaMemcpyAsync(x_right_out, d + o_x, (size_t)n_l * 4, cudaMemcpyDeviceToHost, s));
-    PLP_CUDA_TRY(cudaMemcpyAsync(depths_out, d + o_d, (size_t)n_l * 4, cudaMemcpyDeviceToHost, s));
-    if (best_right_out) PLP_CUDA_TRY(cudaMemcpyAsync(best_right_out, d + o_b, (size_t)n_l * 4, cudaMemcpyDeviceToHost, s));
+    PLP_CUDA_TRY(cudaMemcpyAsync(x_right_out, dx, (size_t)n_l * 4, cudaMemcpyDeviceToHost, s));
+    PLP_CUDA_TRY(cudaMemcpyAsync(depths_out, dd, (size_t)n_l * 4, cudaMemcpyDeviceToHost, s));
+    if (best_right_out) PLP_CUDA_TRY(cudaMemcpyAsync(best_right_out, db, (size_t)n_l * 4, cudaMemcpyDeviceToHost, s));
     PLP_CUDA_TRY(cudaStreamSynchronize(s));
     return PLP_OK;
 }
