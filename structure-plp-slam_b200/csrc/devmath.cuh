@@ -1,5 +1,6 @@
-// devmath.cuh -- small device helpers shared by all kernels (256-bit Hamming, OpenCV rounding, div_up).  Depends only on
-// <stdint.h> and CUDA built-ins, so the kernel headers that include it can also be compiled by tests/cta_emu.
+// devmath.cuh -- small device helpers shared by all kernels (256-bit Hamming, descriptor loads, OpenCV rounding,
+// div_up).  Depends only on <stdint.h> and CUDA built-ins, so the kernel headers that include it can also be compiled by
+// tests/cta_emu.
 #pragma once
 #include <stdint.h>
 
@@ -26,6 +27,13 @@ __device__ __forceinline__ int hamming256(const uint4 a0, const uint4 a1, const 
                                           const uint4 b1) {
     return __popc(a0.x ^ b0.x) + __popc(a0.y ^ b0.y) + __popc(a0.z ^ b0.z) + __popc(a0.w ^ b0.w) +
            __popc(a1.x ^ b1.x) + __popc(a1.y ^ b1.y) + __popc(a1.z ^ b1.z) + __popc(a1.w ^ b1.w);
+}
+
+// one 32-byte descriptor as two read-only 16-byte loads (p must be 16-byte aligned)
+__device__ __forceinline__ void load_desc(const uint8_t *p, uint4 &a, uint4 &b) {
+    const uint4 *q = reinterpret_cast<const uint4 *>(p);
+    a = __ldg(q);
+    b = __ldg(q + 1);
 }
 
 // cvFloor / cvCeil / cvRound for float and double (OpenCV semantics: floor, ceil, round-half-even)

@@ -55,12 +55,6 @@ struct FuseParams {
     int mode;
 };
 
-__device__ __forceinline__ void load_desc(const uint8_t *p, uint4 &a, uint4 &b) {
-    const uint4 *q = reinterpret_cast<const uint4 *>(p);
-    a = __ldg(q);
-    b = __ldg(q + 1);
-}
-
 // data/landmark.cc:341-362 through the host-derived threshold table
 __device__ __forceinline__ int predict_level(float ratio, const FuseParams &P) {
     int lvl = 0;

@@ -8,6 +8,7 @@ namespace plp {
 
 constexpr int kMatchMaxPoints = 3072;  // per-frame keypoint capacity of the window matcher (smem bound)
 constexpr int kBruteMaxPoints = 4096;
+constexpr int kLineMaxLines = 16384;   // per-frame keyline capacity of the keyline matcher (smem bound)
 
 plp_status launch_point_match(plp_ctx *ctx, const PointMatchJob *d_jobs, int num_jobs, int max_n,
                               const plp_grid &grid, int ratio_test, float lowe_ratio,
